@@ -13,6 +13,7 @@ north-star's target shape) with its own clock record: roofline.v128256.
   python bench.py --impl reference ...                    # the reference's CPU algorithm (oracle port)
   python bench.py --workload llama --model 1b|8b ...      # configs[2] / [3]: model in the loop, sharded, one LACB file
   python bench.py --workload stress                       # configs[4]: 8192 streams x vocab 128256, per-token decode
+  python bench.py --dump-outputs DIR ...                  # also the last step's streams and symbols as DIR/*.npy
 
 Under torchrun every rank codes its own 1024 streams (independent chunks shard with no
 data-path collective); the only collective is ONE gather of per-stream bit lengths per job.
@@ -275,6 +276,30 @@ class Job:
         return enc, dec
 
 
+DUMP_BYTES = 64 * 10**6 - 4096   # everything --dump-outputs writes, npy headers included
+
+
+def dump_outputs(path, job):
+    """What the caller of the timed path received in the last step, as path/<name>.npy, so that two builds can be
+    compared output for output: nbits (bits coded per stream), stream_bytes (each stream's ceil(nbits / 8) coded
+    bytes, concatenated in stream order), symbols (the decoded tokens, [streams, tokens]) and stream_index (the
+    streams written: all of them, or a fixed seeded sample of whole streams where all would exceed 64 MB)."""
+    nbits = job.nbits().cpu().numpy()
+    nbytes = (nbits + 7) // 8
+    tokens = job.n_slices * job.T
+    cost = 4 * nbytes + 4 * tokens + 8 + 8
+    order = np.random.default_rng(0).permutation(job.S)
+    keep = np.sort(order[:int(np.searchsorted(np.cumsum(cost[order]), DUMP_BYTES, side="right"))])
+    out = job.out.cpu().numpy()
+    symbols = job.back.permute(1, 0, 2).reshape(job.S, tokens).cpu().numpy()
+    arrays = {"stream_index": keep.astype(np.float64), "nbits": nbits[keep].astype(np.float64),
+              "stream_bytes": np.concatenate([out[s, :nbytes[s]] for s in keep]).astype(np.float32),
+              "symbols": symbols[keep].astype(np.float32)}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def roofline_numbers(rows, V, encode_ms, decode_ms):
     """algorithmic bytes of one call (the logits once, one symbol per row) and the two achieved GB/s figures"""
     alg = rows * (V * 4 + 4)
@@ -341,6 +366,8 @@ def run_gpu(args):
         elapsed_ms = float(t.item())
     clk = clocks.stop() if rank == 0 else None
     job.check()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, job)
     encode_ms, decode_ms = Job.slice_times(evs)
 
     # ---------------- the north-star target shape: vocab 128256 (configs[3] / [4]), same 2.1 GB per slice
@@ -674,6 +701,8 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=4)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the coded streams and decoded symbols of the last timed step (rank 0's) to DIR/*.npy")
     # measurement switches (the driver's contract run uses the defaults = BASELINE.json configs[1])
     ap.add_argument("--vocab", type=int, default=VOCAB)
     ap.add_argument("--streams", type=int, default=STREAMS)
@@ -693,6 +722,10 @@ def main():
     ap.add_argument("--stress-streams", type=int, default=8192)
     ap.add_argument("--stress-tokens", type=int, default=64)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl, args.workload) != ("lac_b200", "coder"):
+        ap.error("--dump-outputs writes the outputs of the coder workload of lac_b200")
     globals().update(VOCAB=args.vocab, STREAMS=args.streams, SLICE=args.slice, CHUNK_TOKENS=args.chunk_tokens)
     if args.impl == "reference":
         run_reference(args)

@@ -64,6 +64,21 @@ def pack_case(store, name, **kw):
         store[f"{name}/{k}"] = np.asarray(v)
 
 
+def save_by_field(path, store, names):
+    """One array per field instead of one per case and field (an npz pays ~200 bytes per member): a scalar field
+    holds one value per case, an array field the cases' arrays concatenated, split at '<field>_off'.
+    tests/conftest.py reads it back keyed '<case>/<field>'."""
+    out = {"names": np.array(names)}
+    for f in sorted({k.split("/", 1)[1] for k in store if "/" in k}):
+        vals = [store[f"{nm}/{f}"] for nm in names]
+        if vals[0].ndim == 0:
+            out[f] = np.array(vals)
+        else:
+            out[f] = np.concatenate(vals)
+            out[f"{f}_off"] = np.cumsum([0] + [len(v) for v in vals]).astype(np.int64)
+    np.savez_compressed(path, **out)
+
+
 # ---------------------------------------------------------------- arith_code: shared small tables
 def gen_ac_small(rng):
     store, names = {}, []
@@ -109,8 +124,7 @@ def gen_ac_small(rng):
                               minp=int(pred.minp), syms=np.array(syms, dtype=np.int32), stop=stop,
                               bits=np.array(bits, dtype=np.uint8), dec=np.array(dec, dtype=np.int32),
                               dec_err=err)
-    store["names"] = np.array(names)
-    np.savez_compressed(os.path.join(HERE, "ac_small.npz"), **store)
+    save_by_field(os.path.join(HERE, "ac_small.npz"), store, names)
     print("ac_small:", len(names), "cases")
 
 

@@ -382,8 +382,8 @@ def _golden(golden_dir, name):
     return np.load(os.path.join(golden_dir, name), allow_pickle=False)
 
 
-def test_golden_ac_small_tables(golden_dir):
-    g = _golden(golden_dir, "ac_small.npz")
+def test_golden_ac_small_tables(ac_small):
+    g = ac_small
     n_checked = n_dec = 0
     for nm in g["names"]:
         prec, stop = int(g[f"{nm}/prec"]), int(g[f"{nm}/stop"])

@@ -66,9 +66,9 @@ needs_gpu = pytest.mark.skipif(not torch.cuda.is_available(), reason="no CUDA de
 
 @gpu
 @needs_gpu
-def test_mirror_ac_on_goldens(golden_dir):
+def test_mirror_ac_on_goldens(ac_small):
     """Every ac_small golden (696 cases): whole-sequence bits / encode, counted decode."""
-    g = np.load(os.path.join(golden_dir, "ac_small.npz"))
+    g = ac_small
     for nm in list(g["names"]):
         prec, stop = int(g[f"{nm}/prec"]), int(g[f"{nm}/stop"])
         dist, syms = [int(x) for x in g[f"{nm}/dist"]], [int(x) for x in g[f"{nm}/syms"]]

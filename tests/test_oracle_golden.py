@@ -22,8 +22,8 @@ def _adaptive_tables(data, V=256):
     return tabs
 
 
-def test_ac_small_encode_and_decode(golden_dir):
-    g = _load(golden_dir, "ac_small.npz")
+def test_ac_small_encode_and_decode(ac_small):
+    g = ac_small
     names = list(g["names"])
     assert len(names) > 500
     n_fudged = 0
