@@ -24,14 +24,18 @@
 //          No F2I anywhere: float->int conversion runs at 16 threads/clk/SM on B200 (measured limiter).
 //   S_w  = sum q_i (< 2^39.5),  c_i = sum of q_j, j < i inside the segment;  summary word = (S_w << 24) | r_w
 // per row:
-//   r    = max r_w;  DEGENERATE (uniform table) when r is EMPTY or POISON
+//   r    = max r_w;  DEGENERATE when r is EMPTY or POISON: cum_i = i, so every symbol but the last gets 2^-32 and the
+//                    last takes the rest (not a uniform table)
 //   d_w  = r - r_w,  W_w = (r_w == 0 || d_w >= 40) ? 0 : S_w >> d_w,  Q = sum W_w
 //   C_i  = sum_{w' < w} W_w' + (c_i >> d_w)
 //   s    = bitlen(Q) - 1,  Qn = Q normalised to [2^31, 2^32),  R = floor(((2^32 - V) << 31) / (Qn + 1))
 //   cum_i = ((C_i * R) >> s) + i,  cum_V = 2^32     => every frequency >= 1
 //
 // Replaces the reference's float table builders (llama_compress.py:24-30, arithmetic_coding.py:57-62); the
-// quantisation differs from theirs by design, bound in DESIGN.md section 3.
+// quantisation differs from theirs by design.  Per element (DESIGN.md section 3, tests/test_lq32_accuracy.py):
+// p_hat_i >= (1 - V/2^32)(1 - 2^-29)[(1 - d)/(1 + d) p_i - 2^-27.5 p_max], d = 1.025e-4, up to the fp32 rounding of
+// log2e, for every element outside an EMPTY segment -- the polynomial's error is in the normaliser Q as well as in
+// the element, so the relative deficit reaches 2d + V/2^32, not d.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>

@@ -484,7 +484,7 @@ static inline uint32_t f2u(float f) { uint32_t u; memcpy(&u, &f, 4); return u; }
  *                                   exponent field of [2^25, 2^26) ends in 00, so four q fit a uint32 sum)
  *   S_w   = sum q_i  (< 2^39.5; 0 for EMPTY / POISON segments),  c_i = sum of q_j over j < i inside the segment
  * per row:
- *   r     = max_w r_w ;  the row is DEGENERATE (every W_w = 0, uniform table) when r is 0 or POISON
+ *   r     = max_w r_w ;  the row is DEGENERATE (every W_w = 0, cum_i = i: not uniform, the last symbol takes the rest) when r is 0 or POISON
  *   d_w   = r - r_w ,  W_w = (r_w == 0 || d_w >= 40) ? 0 : S_w >> d_w ,  Q = sum W_w
  *   C_i   = sum_{w' < w} W_w' + (c_i >> d_w)        (0 instead of the shifted term when W_w is forced to 0)
  *   cum_i = ((C_i * R) >> s) + i  with (R, s) from Q as below,  cum_V = 2^32
