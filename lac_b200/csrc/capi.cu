@@ -9,6 +9,7 @@
 #include <cuda_runtime.h>
 
 #include "launch.h"
+#include "lq32.cuh"
 
 namespace lac {
 cudaError_t launch_status_or(const void* state, int64_t n, int stride_words, int status_word, uint32_t* d_or,
@@ -67,8 +68,7 @@ int lac_device_info(int* sm_count, int* cc_major, int* cc_minor, int64_t* hbm_by
 
 int64_t lac_workspace_bytes(int64_t rows, int32_t vocab) {
     if (rows < 0 || vocab < 1 || vocab > lac::max_vocab()) return 0;
-    int parts = 1;
-    lac::path_for(nullptr, vocab, 0, 0, &parts);
+    const int parts = lq::parts_of(vocab);
     const int64_t chunk = lac::summ_chunk_rows(parts);
     return (int64_t)lac::summ_bytes(rows < chunk ? (rows < 1 ? 1 : rows) : chunk, parts);
 }
@@ -116,8 +116,8 @@ int lac_ac_encode_pairs(const uint32_t* d_pairs, int64_t n_streams, int64_t T, i
         return fail(LAC_E_ARG, "lac_ac_encode_pairs: bad argument");
     if (!prec_ok(prec, 34)) return fail(LAC_E_ARG, "lac_ac_encode_pairs: prec %d outside [34, 60]", prec);
     if ((uintptr_t)d_pairs & 7) return fail(LAC_E_ARG, "lac_ac_encode_pairs: d_pairs must be 8-byte aligned");
-    CK(lac::launch_encode_pairs(d_pairs, n_streams, T, stream_stride, tok_stride, d_ntok, d_state, d_out, out_stride,
-                                finish, prec, (cudaStream_t)stream),
+    CK(lac::launch_encode_pairs(d_pairs, n_streams, T, stream_stride, tok_stride, d_ntok, 0, d_state, d_out,
+                                out_stride, finish, prec, (cudaStream_t)stream),
        "lac_ac_encode_pairs");
     return LAC_OK;
 }

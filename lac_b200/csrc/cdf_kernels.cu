@@ -11,8 +11,9 @@
 // like everything else (LQ32's block form, lq32.cuh, has no row-wide dependency in this pass: no cluster, no DSMEM).
 // Warp w owns segment w of the tile; the tile is read from HBM exactly once and then lives in registers:
 //
-//   staging  the tile arrives as NCH TMA bulk copies (cp.async.bulk; 4 x 32 KB) into a shared-memory ring, each
-//            chunk with its own mbarrier; the warps of a chunk move it to registers.
+//   staging  the tile arrives as 4 TMA bulk copies of 32 KB (cp.async.bulk) into a shared-memory ring, each
+//            chunk with its own mbarrier; the warps of a chunk move it to registers.  Rows that are not 16-byte
+//            aligned or have V % 4 != 0 take scalar loads instead (summary_kernel<1>: no ring, no barrier).
 //   phase A  segment maximum (REDUX) and the ONE barrier of the tile, whose only purpose is the ring: right after
 //            it the chunk leaders re-arm their mbarriers and issue the bulk copies of the CTA's NEXT tile, so
 //            128 KB per SM are in flight during the compute phase.
@@ -31,50 +32,39 @@
 #include "ptx.cuh"
 #include "rowsum.cuh"
 
-#ifndef LAC_DEFAULT_TILE_WARPS
-#define LAC_DEFAULT_TILE_WARPS 32
-#endif
-
 namespace lac {
 
-constexpr int kMaxWarps = 32;
-
-// A tile is TW consecutive segments of a row (TW = 32: one part of the row, one CTA of 1024 threads per SM;
-// TW = 16 / 8: half / quarter parts, 2 / 4 CTAs of 512 / 256 threads per SM whose staging and compute phases
-// interleave).  It arrives as NCH TMA chunks.  Measured on B200 (profiles/microbench/tma_stream.cu): every
+// A tile is one part of a row: 32 consecutive segments, one per warp of a CTA of 1024 threads, one CTA per SM.
+// It arrives as 4 TMA chunks of 8 warps (32 KB).  Measured on B200 (profiles/microbench/tma_stream.cu): every
 // cp.async.bulk costs ~0.2 us of per-SM TMA time regardless of size, so 16 KB chunks cap at 4.7 TB/s while 32 and
-// 64 KB chunks reach 7.1 - 7.2 TB/s with the same 128 KB in flight per SM.
-constexpr int kMaxChunks = 8;
-template <int NCH, int TW>
-struct Ring {
-    static constexpr int kWarpsPerChunk = TW / NCH;
-    static constexpr int kSlotGroups = kPerThread / 4 * 32 * kWarpsPerChunk + 1;  // float4 groups per slot
-    static constexpr int kSlotBytes = kSlotGroups * 16;
-    static constexpr int kRingBytes = NCH * kSlotBytes;
-};
+// 64 KB chunks reach 7.1 - 7.2 TB/s with the same 128 KB in flight per SM; 4 x 32 KB is 0.7 % faster than 2 x 64 KB.
+constexpr int kTileWarps = 32;
+constexpr int kChunks = 4;
+constexpr int kWarpsPerChunk = kTileWarps / kChunks;
+constexpr int kSlotGroups = kPerThread / 4 * 32 * kWarpsPerChunk + 1;  // float4 groups per slot
+constexpr int kSlotBytes = kSlotGroups * 16;
+constexpr int kRingBytes = kChunks * kSlotBytes;
 
-// Everything the pass needs to find tile `tau`: row rho = tau / tpr (row (s, t) = (rho / T, rho % T) at
-// base + s * so + t * st), first segment (tau % tpr) * TW.  Lives in the kernel-parameter constant bank.
+// Everything the pass needs to find tile `tau`: row rho = tau / parts (row (s, t) = (rho / T, rho % T) at
+// base + s * so + t * st), first segment (tau % parts) * 32.  Lives in the kernel-parameter constant bank.
 struct SumParams {
     const float* base;
     int64_t so, st;
     uint32_t T, n_tiles;
     int V, G, parts;
     uint32_t inv_parts;  // ceil(2^31 / parts): floor(m / parts) = (m * inv_parts) >> 31 for m * parts < 2^31
-    uint32_t tpr;        // tiles per row = parts * 32 / TW
-    uint32_t inv_tpr;    // ceil(2^31 / tpr)
     int keep_l2;         // 0: stream with evict-first (the logits are read once); 1: leave them in L2 for a second pass
 };
 
-__shared__ uint64_t g_full[kMaxChunks];  // TMA chunk landed
-__shared__ int g_red[2][kMaxWarps];      // per-warp maxima, written before the tile's barrier (see tile())
+__shared__ uint64_t g_full[kChunks];  // TMA chunk landed
+__shared__ int g_red[2][kTileWarps];  // per-warp maxima, written before the tile's barrier (see tile())
 extern __shared__ __align__(128) unsigned char g_ring[];
 
-template <int VEC, bool TMA, int NCH, int TW>
+// VEC = 4: the TMA ring (rows 16-byte aligned, V % 4 == 0); VEC = 1: scalar loads straight to registers.
+template <int VEC>
 struct TileEngine {
+    static constexpr bool kTma = VEC == 4;
     static constexpr int IT = kPerThread / VEC;
-    static constexpr int kWarpsPerChunk = Ring<NCH, TW>::kWarpsPerChunk;
-    static constexpr int kSlotBytes = Ring<NCH, TW>::kSlotBytes;
 
     static __device__ __forceinline__ int warp() { return threadIdx.x >> 5; }
     static __device__ __forceinline__ int lane() { return threadIdx.x & 31; }
@@ -87,11 +77,11 @@ struct TileEngine {
         return (int)(((uint64_t)m * sp.inv_parts) >> 31);
     }
     static __device__ __forceinline__ uint32_t row_index(const SumParams& sp, uint32_t tau) {
-        return (uint32_t)(((uint64_t)tau * sp.inv_tpr) >> 31);
+        return (uint32_t)(((uint64_t)tau * sp.inv_parts) >> 31);
     }
     // first row-wide segment of tile tau
     static __device__ __forceinline__ int seg0_of(const SumParams& sp, uint32_t tau) {
-        return (int)(tau - row_index(sp, tau) * sp.tpr) * TW;
+        return (int)(tau - row_index(sp, tau) * (uint32_t)sp.parts) * kTileWarps;
     }
     static __device__ __forceinline__ const float* row_of(const SumParams& sp, uint32_t tau) {
         const uint32_t rho = row_index(sp, tau);
@@ -101,14 +91,14 @@ struct TileEngine {
 
     static __device__ void setup() {
         if (threadIdx.x == 0) {
-            for (int i = 0; i < NCH; i++) mbar_init(&g_full[i], 1);
+            for (int i = 0; i < kChunks; i++) mbar_init(&g_full[i], 1);
             fence_mbar_init();
         }
         __syncthreads();
     }
     // chunk leader: arm the chunk's mbarrier and issue its bulk copy for tile tau
     static __device__ __forceinline__ void issue(const SumParams& sp, uint32_t tau) {
-        if (TMA && leader()) {
+        if (kTma && leader()) {
             const int gw0 = seg0_of(sp, tau) + chunk() * kWarpsPerChunk;
             const int g0 = seg(sp, gw0);
             const uint32_t nb = (uint32_t)(seg(sp, gw0 + kWarpsPerChunk) - g0) * 16u;
@@ -131,7 +121,7 @@ struct TileEngine {
             const int s0 = seg0_of(sp, tau);
             const int gw = s0 + warp();
             const int gb = seg(sp, gw), ge = seg(sp, gw + 1), ln = lane();
-            if (TMA) {
+            if (kTma) {
                 const int gw0 = s0 + chunk() * kWarpsPerChunk;
                 const int c0 = seg(sp, gw0);
                 if (seg(sp, gw0 + kWarpsPerChunk) > c0) mbar_wait(&g_full[chunk()], it & 1);
@@ -166,24 +156,11 @@ struct TileEngine {
                 }
             } else {
                 const float* row = row_of(sp, tau);
-                if (VEC == 4) {
+                const int e0 = 4 * gb, e1 = min(sp.V, 4 * ge);
 #pragma unroll
-                    for (int k = 0; k < IT; k++) {
-                        const int g = gb + k * 32 + ln;
-                        float4 v = make_float4(lq::neg_inf(), lq::neg_inf(), lq::neg_inf(), lq::neg_inf());
-                        if (g < ge) v = ldg_stream4(row + 4 * (int64_t)g);
-                        x[4 * k + 0] = v.x;
-                        x[4 * k + 1] = v.y;
-                        x[4 * k + 2] = v.z;
-                        x[4 * k + 3] = v.w;
-                    }
-                } else {
-                    const int e0 = 4 * gb, e1 = min(sp.V, 4 * ge);
-#pragma unroll
-                    for (int k = 0; k < IT; k++) {
-                        const int e = e0 + k * 32 + ln;
-                        x[k] = e < e1 ? ldg_stream1(row + e) : lq::neg_inf();
-                    }
+                for (int k = 0; k < IT; k++) {
+                    const int e = e0 + k * 32 + ln;
+                    x[k] = e < e1 ? ldg_stream1(row + e) : lq::neg_inf();
                 }
             }
         }
@@ -192,7 +169,7 @@ struct TileEngine {
 #pragma unroll
         for (int i = 0; i < kPerThread; i++) m = fmaxf(m, x[i]);
         const int mw = __reduce_max_sync(0xffffffffu, f2ord(m));
-        if (TMA) {
+        if (kTma) {
             // mw depends on every shared-memory load of the warp: storing it before the barrier means that after
             // the barrier the whole tile is in registers and the ring can be overwritten
             if (lane() == 0) *reinterpret_cast<volatile int*>(&g_red[it & 1][warp()]) = mw;
@@ -217,15 +194,15 @@ struct TileEngine {
             lane_sum += (q0 + q1) + (q2 + q3);
         }
         const uint64_t ws = warp_sum48(lane_sum);
-        if (lane() == 0) summ[(uint64_t)tau * TW + warp()] = lq::pack_word(ws, code);
+        if (lane() == 0) summ[(uint64_t)tau * kTileWarps + warp()] = lq::pack_word(ws, code);
     }
 };
 
-template <int VEC, bool TMA, int NCH, int TW>
-__global__ void __launch_bounds__(32 * TW, 32 / TW)
+template <int VEC>
+__global__ void __launch_bounds__(32 * kTileWarps, 1)
 summary_kernel(const __grid_constant__ SumParams sp, uint64_t* __restrict__ summ) {
-    using Eng = TileEngine<VEC, TMA, NCH, TW>;
-    if (TMA) Eng::setup();
+    using Eng = TileEngine<VEC>;
+    if (Eng::kTma) Eng::setup();
     uint32_t tau = blockIdx.x;
     if (tau < sp.n_tiles) Eng::issue(sp, tau);
     for (uint32_t it = 0; tau < sp.n_tiles; tau += gridDim.x, it++) Eng::tile(sp, tau, it, summ);
@@ -354,78 +331,49 @@ int sm_count() {
     return cached[dev];
 }
 
-// Path selection: number of parts (1 .. 8) and the staging path of pass 1:
-// 0: scalar LDG (any alignment, any V), 1: 128-bit LDG, 2 / 4 / 8: TMA bulk ring with that many chunks per tile
-// (default 4; LAC_NO_TMA=1 and LAC_TMA_CHUNKS=n are measurement switches).  -1: unsupported.
+// Number of parts (1 .. 8) and the load width of pass 1 and the second passes: 4 for 16-byte aligned rows with
+// V % 4 == 0 (the TMA ring, float4 loads), 1 for anything else (scalar loads), -1 if V is unsupported.
 int path_for(const float* p, int V, int64_t s0, int64_t s1, int* parts) {
     *parts = lq::parts_of(V);
     if (V < 1 || *parts > lq::kMaxParts) return -1;
     const bool v4 = (V % 4 == 0) && ((((uintptr_t)p) & 15) == 0) && (s0 % 4 == 0) && (s1 % 4 == 0);
-    if (!v4) return 0;
-    static const bool no_tma = getenv("LAC_NO_TMA") != nullptr;
-    if (no_tma) return 1;
-    static const int nch = getenv("LAC_TMA_CHUNKS") ? atoi(getenv("LAC_TMA_CHUNKS")) : 4;
-    return (nch == 2 || nch == 8) ? nch : 4;  // 4 x 32 KB: 0.7 % faster than 2 x 64 KB with one barrier per tile
-}
-
-template <int TW, typename K>
-static cudaError_t launch_ring(K kernel, int ring_bytes, SumParams sp, uint64_t* summ, cudaStream_t st) {
-    sp.tpr = (uint32_t)(sp.parts * (32 / TW));
-    sp.inv_tpr = (uint32_t)(((1ull << 31) + sp.tpr - 1) / sp.tpr);
-    sp.n_tiles *= (uint32_t)(32 / TW);
-    if (ring_bytes > 0) {
-        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ring_bytes);
-        if (e != cudaSuccess) return e;
-    }
-    const uint32_t slots = (uint32_t)sm_count() * (32 / TW);
-    const unsigned grid = sp.n_tiles < slots ? sp.n_tiles : slots;
-    kernel<<<grid, 32 * TW, ring_bytes, st>>>(sp, summ);
-    return cudaGetLastError();
-}
-
-// Warps per tile / CTA: 32 (one CTA per SM), 16 or 8 (2 / 4 CTAs per SM).  LAC_TILE_WARPS is a measurement switch.
-static int tile_warps() {
-    static const int tw = getenv("LAC_TILE_WARPS") ? atoi(getenv("LAC_TILE_WARPS")) : LAC_DEFAULT_TILE_WARPS;
-    return (tw == 8 || tw == 16) ? tw : 32;
+    return v4 ? 4 : 1;
 }
 
 // Row summaries of rows (s, t), s < n_outer, t < T, at base + s * so + t * st; summary of row (s, t) at
 // summ + (s * T + t) * 32 * parts.  n_outer * T * parts must stay below 2^26 (summ_rows_for sees to it).
 cudaError_t launch_summary(const float* base, int64_t n_outer, int64_t T, int64_t so, int64_t st_, int V, int parts,
-                           int path, int keep_l2, uint64_t* summ, cudaStream_t st) {
+                           int vec, int keep_l2, uint64_t* summ, cudaStream_t st) {
     SumParams sp;
     sp.base = base;
     sp.so = so;
     sp.st = st_;
     sp.T = (uint32_t)T;
-    sp.n_tiles = (uint32_t)(n_outer * T * parts);  // in parts; launch_ring scales it to tiles of TW warps
+    sp.n_tiles = (uint32_t)(n_outer * T * parts);
     sp.V = V;
     sp.G = lq::groups_of(V);
     sp.parts = parts;
     sp.inv_parts = (uint32_t)(((1ull << 31) + parts - 1) / parts);
-    sp.tpr = sp.inv_tpr = 0;
     sp.keep_l2 = keep_l2;
     if (sp.n_tiles == 0) return cudaSuccess;
-    const int tw = tile_warps();
-    // chunks of 8 warps (32 KB) unless LAC_TMA_CHUNKS asks otherwise (TW = 32 only)
-    if (path >= 2 && tw == 16) return launch_ring<16>(summary_kernel<4, true, 2, 16>, Ring<2, 16>::kRingBytes, sp, summ, st);
-    if (path >= 2 && tw == 8) return launch_ring<8>(summary_kernel<4, true, 1, 8>, Ring<1, 8>::kRingBytes, sp, summ, st);
-    switch (path) {
-        case 2: return launch_ring<32>(summary_kernel<4, true, 2, 32>, Ring<2, 32>::kRingBytes, sp, summ, st);
-        case 4: return launch_ring<32>(summary_kernel<4, true, 4, 32>, Ring<4, 32>::kRingBytes, sp, summ, st);
-        case 8: return launch_ring<32>(summary_kernel<4, true, 8, 32>, Ring<8, 32>::kRingBytes, sp, summ, st);
-        case 1: return launch_ring<32>(summary_kernel<4, false, 4, 32>, 0, sp, summ, st);
-        case 0: return launch_ring<32>(summary_kernel<1, false, 4, 32>, 0, sp, summ, st);
-        default: return cudaErrorInvalidValue;
+    const int ring_bytes = vec == 4 ? kRingBytes : 0;
+    void (*kernel)(SumParams, uint64_t*) = vec == 4 ? summary_kernel<4> : summary_kernel<1>;
+    if (ring_bytes > 0) {
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ring_bytes);
+        if (e != cudaSuccess) return e;
     }
+    const uint32_t sms = (uint32_t)sm_count();
+    const unsigned grid = sp.n_tiles < sms ? sp.n_tiles : sms;
+    kernel<<<grid, 32 * kTileWarps, ring_bytes, st>>>(sp, summ);
+    return cudaGetLastError();
 }
 
 // Rows of summary a launch may cover: the scratch budget (LAC_SUMMARY_BYTES: test switch, forces many small
-// chunks) and the tile index (the mul-shift division by the tiles per row is exact below 2^28 tiles).
+// chunks) and the tile index (the mul-shift division by parts is exact below 2^28 tiles).
 int64_t summ_chunk_rows(int parts) {
     static const int64_t budget = getenv("LAC_SUMMARY_BYTES") ? atoll(getenv("LAC_SUMMARY_BYTES")) : (64ll << 20);
     int64_t rows = budget / (32 * parts * 8 + 8);
-    const int64_t lim = ((1ll << 26) - 1) / (parts * 4);  // tiles per row <= 4 * parts
+    const int64_t lim = ((1ll << 26) - 1) / (parts * 4);  // room for 4 tiles per part; changing it moves chunk bounds
     if (rows > lim) rows = lim;
     return rows < 1 ? 1 : rows;
 }
@@ -468,14 +416,14 @@ cudaError_t scratch_put(Scratch* sc, cudaStream_t st) {
     return cudaSuccess;
 }
 
-cudaError_t launch_pairs_status(const float* logits, int64_t n, int64_t T, int64_t so, int64_t st_, int V, int parts,
-                                int path, const uint64_t* summ, const int32_t* syms, int64_t sym_stride,
-                                uint32_t* pairs, uint32_t* status, cudaStream_t st) {
+cudaError_t launch_pairs(const float* logits, int64_t n, int64_t T, int64_t so, int64_t st_, int V, int parts, int vec,
+                         const uint64_t* summ, const int32_t* syms, int64_t sym_stride, uint32_t* pairs,
+                         uint32_t* status, cudaStream_t st) {
     const int64_t rows = n * T;
     if (rows == 0) return cudaSuccess;
     const unsigned blocks = (unsigned)((rows + 7) / 8);
 #define LAC_PAIR(CL_)                                                                                                 \
-    if (path == 0)                                                                                                    \
+    if (vec == 1)                                                                                                     \
         pair_kernel<1, CL_><<<blocks, 256, 0, st>>>(logits, rows, T, so, st_, V, summ, syms, sym_stride, pairs, status); \
     else                                                                                                              \
         pair_kernel<4, CL_><<<blocks, 256, 0, st>>>(logits, rows, T, so, st_, V, summ, syms, sym_stride, pairs, status)
@@ -483,19 +431,14 @@ cudaError_t launch_pairs_status(const float* logits, int64_t n, int64_t T, int64
 #undef LAC_PAIR
     return cudaGetLastError();
 }
-cudaError_t launch_pairs(const float* logits, int64_t n, int64_t T, int64_t so, int64_t st_, int V, int parts, int path,
-                         const uint64_t* summ, const int32_t* syms, int64_t sym_stride, uint32_t* pairs,
-                         cudaStream_t st) {
-    return launch_pairs_status(logits, n, T, so, st_, V, parts, path, summ, syms, sym_stride, pairs, nullptr, st);
-}
 
 // lac_cdf_lookup_f32: summary pass + one warp per row for the pair.
 cudaError_t launch_lookup(const float* logits, int64_t rows, int V, int64_t row_stride, const int32_t* syms,
                           uint32_t* pairs, uint32_t* status, void* ws, size_t ws_bytes, cudaStream_t st) {
     if (rows == 0) return cudaSuccess;
     int parts = 1;
-    const int path = path_for(logits, V, row_stride, 0, &parts);
-    if (path < 0) return cudaErrorInvalidValue;
+    const int vec = path_for(logits, V, row_stride, 0, &parts);
+    if (vec < 0) return cudaErrorInvalidValue;
     const int64_t chunk = summ_rows_for(rows, parts, ws, ws_bytes);
     Scratch sc;
     cudaError_t e = scratch_get(&sc, summ_bytes(chunk, parts), ws, ws_bytes, st);
@@ -504,10 +447,10 @@ cudaError_t launch_lookup(const float* logits, int64_t rows, int V, int64_t row_
     for (int64_t r0 = 0; r0 < rows && e == cudaSuccess; r0 += chunk) {
         const int64_t rn = rows - r0 < chunk ? rows - r0 : chunk;
         const float* base = logits + r0 * row_stride;
-        e = launch_summary(base, rn, 1, row_stride, 0, V, parts, path, 0, summ, st);
+        e = launch_summary(base, rn, 1, row_stride, 0, V, parts, vec, 0, summ, st);
         if (e != cudaSuccess) break;
-        e = launch_pairs_status(base, rn, 1, row_stride, 0, V, parts, path, summ, syms + r0, 1, pairs + 2 * r0,
-                                status ? status + r0 : nullptr, st);
+        e = launch_pairs(base, rn, 1, row_stride, 0, V, parts, vec, summ, syms + r0, 1, pairs + 2 * r0,
+                         status ? status + r0 : nullptr, st);
         if (e != cudaSuccess) break;
         e = cudaGetLastError();
     }
@@ -521,8 +464,8 @@ cudaError_t launch_build(const float* logits, int64_t rows, int V, int64_t row_s
                          size_t ws_bytes, cudaStream_t st) {
     if (rows == 0) return cudaSuccess;
     int parts = 1;
-    const int path = path_for(logits, V, row_stride, 0, &parts);
-    if (path < 0) return cudaErrorInvalidValue;
+    const int vec = path_for(logits, V, row_stride, 0, &parts);
+    if (vec < 0) return cudaErrorInvalidValue;
     int64_t l2rows = (32ll << 20) / ((int64_t)V * 4);
     l2rows = l2rows < 1 ? 1 : (l2rows > rows ? rows : l2rows);
     const int64_t chunk = summ_rows_for(l2rows, parts, ws, ws_bytes);
@@ -533,11 +476,11 @@ cudaError_t launch_build(const float* logits, int64_t rows, int V, int64_t row_s
     for (int64_t r0 = 0; r0 < rows && e == cudaSuccess; r0 += chunk) {
         const int64_t rn = rows - r0 < chunk ? rows - r0 : chunk;
         const float* base = logits + r0 * row_stride;
-        e = launch_summary(base, rn, 1, row_stride, 0, V, parts, path, 1, summ, st);
+        e = launch_summary(base, rn, 1, row_stride, 0, V, parts, vec, 1, summ, st);
         if (e != cudaSuccess) break;
         const unsigned blocks = (unsigned)((rn * 32 * parts + 7) / 8);
 #define LAC_TABLE(CL_)                                                                                          \
-    if (path == 0) table_kernel<1, CL_><<<blocks, 256, 0, st>>>(base, rn, row_stride, V, summ, cum + r0 * (int64_t)V); \
+    if (vec == 1) table_kernel<1, CL_><<<blocks, 256, 0, st>>>(base, rn, row_stride, V, summ, cum + r0 * (int64_t)V); \
     else table_kernel<4, CL_><<<blocks, 256, 0, st>>>(base, rn, row_stride, V, summ, cum + r0 * (int64_t)V)
         LAC_BY_PARTS(parts, LAC_TABLE)
 #undef LAC_TABLE

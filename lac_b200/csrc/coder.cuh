@@ -237,6 +237,24 @@ __device__ __forceinline__ void ac_narrow32(int64_t& l, int64_t& h, uint32_t lo,
     l += (int64_t)r0;
 }
 
+// One token of A_to_bin on a (lo, hi) pair of the lookup: narrow, renormalise, append the k bits.  Returns false,
+// coding nothing, when the stream must stop.  A pair with hi != 0 && hi <= lo codes no interval:
+// (0xFFFFFFFF, 0xFFFFFFFF) is the lookup's sentinel for a symbol outside [0, V) -> LAC_ST_SYMBOL (the reference
+// raises "unknown symbol", arith_code.py:100-101), any other such pair is a zero-width symbol -> LAC_ST_TABLE (the
+// reference would never terminate).  A stream that is already truncated (LAC_ST_CAP) codes nothing more.
+template <class Writer>
+__device__ __forceinline__ bool code_pair(int64_t& l, int64_t& h, uint2 pr, int P, Writer& bw) {
+    if (pr.y != 0 && pr.y <= pr.x) {
+        bw.status |= (pr.x == 0xFFFFFFFFu && pr.y == 0xFFFFFFFFu) ? LAC_ST_SYMBOL : LAC_ST_TABLE;
+        return false;
+    }
+    if (bw.status & LAC_ST_CAP) return false;
+    ac_narrow32(l, h, pr.x, pr.y);
+    const int k = renorm_count((uint64_t)(h - l + 1), P);
+    bw.append(renorm_apply(l, h, P, k), k);
+    return true;
+}
+
 __device__ __forceinline__ int64_t region_overlap(int64_t a, int64_t b, int64_t c, int64_t d) {
     int64_t lo = a > c ? a : c, hi = b < d ? b : d;
     int64_t v = hi - lo + 1;

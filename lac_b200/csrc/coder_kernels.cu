@@ -1,10 +1,9 @@
 // coder_kernels.cu -- batched multi-stream range coder kernels (north-star part (b)).
 //
-//   encode_pairs_staged_kernel   one lane per stream, a few streams per warp; (lo, hi) pairs on the fixed total
+//   encode_pairs_staged_kernel   one lane per stream, 4 streams per warp; (lo, hi) pairs on the fixed total
 //                         2^32 (output of the lookup) -> MSB-first bytes.  low / high live in registers, the k
 //                         renormalisation bits of a token are appended in one step with carry resolution
 //                         (coder.cuh) into a shared-memory stage that the whole warp flushes.
-//   encode_pairs_kernel   the same coder with one thread per stream and direct byte stores (measurement switch)
 //   encode_fused_kernel   symbol ranges + coder in one launch for the model-in-the-loop step (T <= 4)
 //   ac_tables_*           one warp per stream; int64 inclusive cumulative tables exactly as
 //                         CDFPredictor.dist holds them, including fudged_dist
@@ -16,16 +15,11 @@
 //                         Llama_AC, flag LAC_F_WRAP64).
 //   acs_tables_*          ACSampler / Region semantics (arithmetic_coding.py).
 #include <cstdint>
-#include <cstdlib>
 #include <cuda_runtime.h>
 
 #include "coder.cuh"
 #include "launch.h"
 #include "rowsum.cuh"
-
-#ifndef LAC_DEFAULT_CODER_SPB
-#define LAC_DEFAULT_CODER_SPB 4
-#endif
 
 namespace lac {
 
@@ -54,77 +48,25 @@ __device__ __forceinline__ int64_t warp_sum_i64(int64_t v) {
 }
 
 // ------------------------------------------------------------------ pairs encoder
-__global__ void encode_pairs_kernel(const uint2* __restrict__ pairs, int64_t n_streams, int64_t T,
-                                    int64_t stream_stride, int64_t tok_stride, const int32_t* __restrict__ ntok,
-                                    int64_t t0, lac_enc_state* __restrict__ state, uint8_t* __restrict__ out,
-                                    int64_t out_stride, int finish, int P) {
-    int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    int64_t l = state[s].low, h = state[s].high;
-    coder::BitWriter bw;
-    bw.open(out + s * out_stride, (uint64_t)out_stride, state[s].nbits);
-    bw.status = state[s].status;
-    int64_t Ts = T;  // ntok counts from t0 tokens before the first pair of this call
-    if (ntok) {
-        Ts = (int64_t)ntok[s] - t0;
-        Ts = Ts < 0 ? 0 : (Ts > T ? T : Ts);
-    }
-    const uint2* p = pairs + s * stream_stride;
-    // the pairs of a stream are T * 8 bytes apart from the next stream's, so every load is its own memory
-    // transaction: fetch them eight tokens at a time (independent loads in flight together), then code serially
-    constexpr int kBatch = 8;
-    bool bad = false;
-    for (int64_t t0 = 0; t0 < Ts && !bad; t0 += kBatch) {
-        uint2 pr[kBatch];
-#pragma unroll
-        for (int j = 0; j < kBatch; j++) {
-            const int64_t t = t0 + j < Ts ? t0 + j : Ts - 1;
-            pr[j] = p[t * tok_stride];
-        }
-#pragma unroll
-        for (int j = 0; j < kBatch; j++) {
-            if (t0 + j < Ts && !bad) {
-                if (pr[j].y != 0 && pr[j].y <= pr[j].x) {
-                    // the lookup's sentinel for a symbol outside [0, V) (the reference raises "unknown symbol",
-                    // arith_code.py:100-101), or a zero-width symbol (the reference would never terminate)
-                    bw.status |= (pr[j].x == 0xFFFFFFFFu && pr[j].y == 0xFFFFFFFFu) ? LAC_ST_SYMBOL : LAC_ST_TABLE;
-                    bad = true;
-                } else if (bw.status & LAC_ST_CAP) {
-                    bad = true;  // truncated: stop coding this stream
-                } else {
-                    coder::ac_narrow32(l, h, pr[j].x, pr[j].y);
-                    int k = coder::renorm_count((uint64_t)(h - l + 1), P);
-                    int64_t E = coder::renorm_apply(l, h, P, k);
-                    bw.append(E, k);
-                }
-            }
-        }
-    }
-    if (finish && !(bw.status & (LAC_ST_TABLE | LAC_ST_SYMBOL | LAC_ST_CAP))) coder::ac_flush(l, h, P, bw);
-    bw.close();
-    state[s].low = l;
-    state[s].high = h;
-    state[s].nbits = bw.nbits;
-    state[s].status = bw.status;
-}
-
-// ------------------------------------------------------------------ pairs encoder with warp-aggregated output
-// One warp per `spb` streams (lanes 0 .. spb-1 run A_to_bin, low / high in registers).  The bytes of a batch of 16
-// tokens go to a per-stream shared-memory stage (coder::StagedWriter: carries resolved there); after every batch
-// the WHOLE warp copies the stages to the streams' global buffers -- 32 consecutive bytes of one stream per store
-// instruction instead of one byte per store and lane.
-constexpr int kStagedMaxSpb = 16;
+// One warp per kPairsSpb streams (lanes 0 .. kPairsSpb-1 run A_to_bin, low / high in registers).  The bytes of a
+// batch of 16 tokens go to a per-stream shared-memory stage (coder::StagedWriter: carries resolved there); after
+// every batch the WHOLE warp copies the stages to the streams' global buffers -- 32 consecutive bytes of one stream
+// per store instruction instead of one byte per store and lane.  Each coder lane is a long dependent chain with
+// data-dependent inner loops (bits per token differ per stream), so few streams per warp (less divergence) on many
+// SMs (more schedulers) beat dense blocks.  Measured per [1024 x 16] slice inside the encode call (B200): 2 / 4 / 8
+// streams per warp 0.347 / 0.348 / 0.350 ms, the same as one thread per stream with byte stores: 0.348 ms.
+constexpr int kPairsSpb = 4;
 __global__ void __launch_bounds__(32)
 encode_pairs_staged_kernel(const uint2* __restrict__ pairs, int64_t n_streams, int64_t T, int64_t stream_stride,
                            int64_t tok_stride, const int32_t* __restrict__ ntok, int64_t t0,
                            lac_enc_state* __restrict__ state, uint8_t* __restrict__ out, int64_t out_stride,
-                           int finish, int P, int spb) {
-    __shared__ uint8_t s_stage[kStagedMaxSpb][coder::StagedWriter::kStage + 1];
-    __shared__ unsigned long long s_base[kStagedMaxSpb];
-    __shared__ int s_fill[kStagedMaxSpb];
+                           int finish, int P) {
+    __shared__ uint8_t s_stage[kPairsSpb][coder::StagedWriter::kStage + 1];
+    __shared__ unsigned long long s_base[kPairsSpb];
+    __shared__ int s_fill[kPairsSpb];
     const int lane = threadIdx.x;
-    const int64_t s0 = (int64_t)blockIdx.x * spb;
-    const int ns = (int)min((int64_t)spb, n_streams - s0);
+    const int64_t s0 = (int64_t)blockIdx.x * kPairsSpb;
+    const int ns = (int)min((int64_t)kPairsSpb, n_streams - s0);
     const bool is_coder = lane < ns;
     const int64_t s = s0 + lane;
     int64_t l = 0, h = 0, Ts = 0;
@@ -155,23 +97,8 @@ encode_pairs_staged_kernel(const uint2* __restrict__ pairs, int64_t n_streams, i
                     pr[j] = p[t * tok_stride];
                 }
 #pragma unroll
-                for (int j = 0; j < kBatch; j++) {
-                    if (tq + j < Ts && !bad) {
-                        if (pr[j].y != 0 && pr[j].y <= pr[j].x) {
-                            // the lookup's sentinel for a symbol outside [0, V) (the reference raises "unknown symbol",
-                            // arith_code.py:100-101), or a zero-width symbol (the reference would never terminate)
-                            bw.status |= (pr[j].x == 0xFFFFFFFFu && pr[j].y == 0xFFFFFFFFu) ? LAC_ST_SYMBOL : LAC_ST_TABLE;
-                            bad = true;
-                        } else if (bw.status & LAC_ST_CAP) {
-                            bad = true;  // truncated: stop coding this stream
-                        } else {
-                            coder::ac_narrow32(l, h, pr[j].x, pr[j].y);
-                            const int k = coder::renorm_count((uint64_t)(h - l + 1), P);
-                            const int64_t E = coder::renorm_apply(l, h, P, k);
-                            bw.append(E, k);
-                        }
-                    }
-                }
+                for (int j = 0; j < kBatch; j++)
+                    if (tq + j < Ts && !bad) bad = !coder::code_pair(l, h, pr[j], P, bw);
             }
             if (last) {
                 if (finish && !(bw.status & (LAC_ST_TABLE | LAC_ST_SYMBOL | LAC_ST_CAP))) coder::ac_flush(l, h, P, bw);
@@ -271,19 +198,8 @@ encode_fused_kernel(const __grid_constant__ EncParams ep) {
         if (is_coder && !dead) {
             const int n_here = min(nt, my_tokens - (int)tb0);
             for (int ti = 0; ti < n_here; ti++) {
-                const uint2 pr = s_pairs[threadIdx.x * nt + ti];
-                if (pr.y != 0 && pr.y <= pr.x) {
-                    // the lookup's sentinel for an unknown symbol (the reference raises, arith_code.py:100-101), or a
-                    // zero-width symbol (the reference would never terminate)
-                    bw.status |= (pr.x == 0xFFFFFFFFu && pr.y == 0xFFFFFFFFu) ? LAC_ST_SYMBOL : LAC_ST_TABLE;
-                    dead = true;
-                    break;
-                }
-                coder::ac_narrow32(l, h, pr.x, pr.y);
-                const int k = coder::renorm_count((uint64_t)(h - l + 1), ep.P);
-                const int64_t E = coder::renorm_apply(l, h, ep.P, k);
-                bw.append(E, k);
-                if (bw.status & LAC_ST_CAP) {
+                // a stream stops at the token that truncates it
+                if (!coder::code_pair(l, h, s_pairs[threadIdx.x * nt + ti], ep.P, bw) || (bw.status & LAC_ST_CAP)) {
                     dead = true;
                     break;
                 }
@@ -740,51 +656,30 @@ cudaError_t launch_enc_init(lac_enc_state* state, int64_t n, int P, cudaStream_t
     return cudaGetLastError();
 }
 
+// ntok counts tokens from t0 tokens before the first pair of the call
 cudaError_t launch_encode_pairs(const uint32_t* pairs, int64_t n, int64_t T, int64_t ss, int64_t ts,
-                                const int32_t* ntok, lac_enc_state* state, uint8_t* out, int64_t out_stride,
-                                int finish, int P, cudaStream_t st) {
-    return launch_encode_pairs_at(pairs, n, T, ss, ts, ntok, 0, state, out, out_stride, finish, P, st);
-}
-cudaError_t launch_encode_pairs_at(const uint32_t* pairs, int64_t n, int64_t T, int64_t ss, int64_t ts,
-                                   const int32_t* ntok, int64_t t0, lac_enc_state* state, uint8_t* out,
-                                   int64_t out_stride, int finish, int P, cudaStream_t st) {
+                                const int32_t* ntok, int64_t t0, lac_enc_state* state, uint8_t* out,
+                                int64_t out_stride, int finish, int P, cudaStream_t st) {
     if (n == 0) return cudaSuccess;
-    // Each coder lane is a long dependent chain with data-dependent inner loops (bits per token differ per stream),
-    // so few streams per warp (less divergence) on many SMs (more schedulers) beat dense blocks.
-    // Default: the staged kernel, 4 streams per warp, warp-wide flushes (LAC_CODER_SPB=n, 1 .. 16).  Measured per
-    // [1024 x 16] slice inside the encode call: 2 / 4 / 8 streams per warp 0.347 / 0.348 / 0.350 ms, the same as the
-    // thread-per-stream kernel with byte stores (LAC_CODER_SPB=0; LAC_CODER_TPB threads per block, default 2): 0.348 ms.
-    static const int spb_env = getenv("LAC_CODER_SPB") ? atoi(getenv("LAC_CODER_SPB")) : LAC_DEFAULT_CODER_SPB;
-    if (spb_env > 0) {
-        const int spb = spb_env > kStagedMaxSpb ? kStagedMaxSpb : spb_env;
-        encode_pairs_staged_kernel<<<(unsigned)((n + spb - 1) / spb), 32, 0, st>>>(
-            reinterpret_cast<const uint2*>(pairs), n, T, ss, ts, ntok, t0, state, out, out_stride, finish, P, spb);
-        return cudaGetLastError();
-    }
-    static const int tpb_env = getenv("LAC_CODER_TPB") ? atoi(getenv("LAC_CODER_TPB")) : 2;
-    const int tpb = tpb_env < 1 ? 1 : (tpb_env > 1024 ? 1024 : tpb_env);
-    encode_pairs_kernel<<<(unsigned)((n + tpb - 1) / tpb), tpb, 0, st>>>(reinterpret_cast<const uint2*>(pairs), n, T, ss,
-                                                                  ts, ntok, t0, state, out, out_stride, finish, P);
+    encode_pairs_staged_kernel<<<(unsigned)((n + kPairsSpb - 1) / kPairsSpb), 32, 0, st>>>(
+        reinterpret_cast<const uint2*>(pairs), n, T, ss, ts, ntok, t0, state, out, out_stride, finish, P);
     return cudaGetLastError();
 }
 
 // lac_ac_encode_logits_f32: per token chunk (the scratch bounds it) the summary pass, then
 //   T <= 4 (the model-in-the-loop step): ONE fused kernel (symbol ranges + coder, pairs in shared memory);
 //   longer slices: pair_kernel over all rows at once (thousands of independent warps, ~20 us per 16k rows) into
-//   the scratch, then the thread-per-stream coder.  A fused kernel keeps 8 warps of registers resident per stream
-//   for the whole serial coding chain -- measured 52 us per [1024 x 16] slice against 37 us for the two kernels.
-cudaError_t launch_pairs(const float* logits, int64_t n, int64_t T, int64_t ss, int64_t ts, int V, int parts, int path,
-                         const uint64_t* summ, const int32_t* syms, int64_t sym_stride, uint32_t* pairs,
-                         cudaStream_t st);  // cdf_kernels.cu
-
+//   the scratch, then the pairs coder (encode_pairs_staged_kernel).  A fused kernel keeps 8 warps of registers
+//   resident per stream for the whole serial coding chain -- measured 52 us per [1024 x 16] slice against 37 us for
+//   the two kernels.
 cudaError_t launch_encode_logits(const float* logits, int64_t n, int64_t T, int64_t ss, int64_t ts, int V,
                                  const int32_t* syms, int64_t sym_stride, const int32_t* ntok, lac_enc_state* state,
                                  uint8_t* out, int64_t out_stride, int finish, int P, void* ws, size_t ws_bytes,
                                  cudaStream_t st) {
     if (n == 0) return cudaSuccess;
     int parts = 1;
-    const int path = path_for(logits, V, ss, ts, &parts);
-    if (path < 0) return cudaErrorInvalidValue;
+    const int vec = path_for(logits, V, ss, ts, &parts);
+    if (vec < 0) return cudaErrorInvalidValue;
     const int64_t Tn = T < 1 ? 1 : T;
     int64_t tc = summ_rows_for(n * Tn, parts, ws, ws_bytes) / n;
     tc = tc < 1 ? 1 : (tc > Tn ? Tn : tc);
@@ -796,14 +691,15 @@ cudaError_t launch_encode_logits(const float* logits, int64_t n, int64_t T, int6
     for (int64_t t0 = 0; (t0 < T || (T == 0 && t0 == 0)) && e == cudaSuccess; t0 += tc) {
         const int64_t tn = T - t0 < tc ? T - t0 : tc;
         const float* base = logits + t0 * ts;
-        if (tn > 0) e = launch_summary(base, n, tn, ss, ts, V, parts, path, 0, (uint64_t*)sc.p, st);
+        if (tn > 0) e = launch_summary(base, n, tn, ss, ts, V, parts, vec, 0, (uint64_t*)sc.p, st);
         if (e != cudaSuccess) break;
         const int fin = (finish && t0 + tn >= T) ? 1 : 0;
         if (!fused) {
-            e = launch_pairs(base, n, tn, ss, ts, V, parts, path, (const uint64_t*)sc.p, syms + t0, sym_stride, pairs, st);
+            e = launch_pairs(base, n, tn, ss, ts, V, parts, vec, (const uint64_t*)sc.p, syms + t0, sym_stride, pairs,
+                             nullptr, st);
             if (e != cudaSuccess) break;
             // ntok counts from the start of the call: shift it by t0 inside the kernel
-            e = launch_encode_pairs_at(pairs, n, tn, tn, 1, ntok, t0, state, out, out_stride, fin, P, st);
+            e = launch_encode_pairs(pairs, n, tn, tn, 1, ntok, t0, state, out, out_stride, fin, P, st);
             continue;
         }
         EncParams ep;
@@ -829,7 +725,7 @@ cudaError_t launch_encode_logits(const float* logits, int64_t n, int64_t T, int6
         if (tn == 0) ep.spb = kEncMaxSpb;  // flush-only call: as many streams per block as the stage allows
         const unsigned blocks = (unsigned)((n + ep.spb - 1) / ep.spb);
 #define LAC_ENC(CL_)                                                             \
-    if (path == 0) encode_fused_kernel<1, CL_><<<blocks, kEncWarps * 32, 0, st>>>(ep); \
+    if (vec == 1) encode_fused_kernel<1, CL_><<<blocks, kEncWarps * 32, 0, st>>>(ep);  \
     else encode_fused_kernel<4, CL_><<<blocks, kEncWarps * 32, 0, st>>>(ep)
         LAC_BY_PARTS(parts, LAC_ENC)
 #undef LAC_ENC

@@ -249,8 +249,8 @@ cudaError_t launch_decode(const float* logits, int64_t n_streams, int64_t T, int
                           int P, void* ws, size_t ws_bytes, cudaStream_t st) {
     if (n_streams == 0 || T == 0) return cudaSuccess;
     int parts = 1;
-    const int path = path_for(logits, V, stream_stride, tok_stride, &parts);
-    if (path < 0) return cudaErrorInvalidValue;
+    const int vec = path_for(logits, V, stream_stride, tok_stride, &parts);
+    if (vec < 0) return cudaErrorInvalidValue;
     int64_t tc = summ_rows_for(n_streams * T, parts, ws, ws_bytes) / n_streams;
     tc = tc < 1 ? 1 : (tc > T ? T : tc);
     Scratch sc;
@@ -261,11 +261,11 @@ cudaError_t launch_decode(const float* logits, int64_t n_streams, int64_t T, int
     for (int64_t t0 = 0; t0 < T && e == cudaSuccess; t0 += tc) {
         const int64_t tn = T - t0 < tc ? T - t0 : tc;
         const float* base = logits + t0 * tok_stride;
-        e = launch_summary(base, n_streams, tn, stream_stride, tok_stride, V, parts, path, 0, summ, st);
+        e = launch_summary(base, n_streams, tn, stream_stride, tok_stride, V, parts, vec, 0, summ, st);
         if (e != cudaSuccess) break;
         const SerialParams rp{base, n_streams, tn, stream_stride, tok_stride, ntok, t0};
 #define LAC_SERIAL(CL_)                                                                                             \
-    if (path == 0)                                                                                                  \
+    if (vec == 1)                                                                                                   \
         decode_serial_kernel<1, CL_><<<serial_blocks, 128, 0, st>>>(rp, V, summ, state, bytes, offsets, syms + t0,   \
                                                                     sym_stride, P);                                 \
     else                                                                                                            \

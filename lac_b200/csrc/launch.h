@@ -18,13 +18,16 @@ cudaError_t scratch_put(Scratch* sc, cudaStream_t st);
 
 int sm_count();
 int max_vocab();
-int path_for(const float* p, int V, int64_t s0, int64_t s1, int* parts);
+int path_for(const float* p, int V, int64_t s0, int64_t s1, int* parts);  // load width: 4, 1 (or -1: unsupported)
 int64_t summ_chunk_rows(int parts);
 int64_t summ_rows_for(int64_t want, int parts, const void* ws, size_t ws_bytes);
 size_t summ_bytes(int64_t rows, int parts);       // scratch per launch: row summaries + (lo, hi) pairs
 size_t summ_only_bytes(int64_t rows, int parts);  // offset of the pairs inside it
 cudaError_t launch_summary(const float* base, int64_t n_outer, int64_t T, int64_t so, int64_t st_, int V, int parts,
-                           int path, int keep_l2, uint64_t* summ, cudaStream_t st);
+                           int vec, int keep_l2, uint64_t* summ, cudaStream_t st);
+cudaError_t launch_pairs(const float* logits, int64_t n, int64_t T, int64_t so, int64_t st_, int V, int parts, int vec,
+                         const uint64_t* summ, const int32_t* syms, int64_t sym_stride, uint32_t* pairs,
+                         uint32_t* status, cudaStream_t st);
 
 // instantiate MACRO(CL) for the run-time number of parts (1 .. 8)
 #define LAC_BY_PARTS(parts, MACRO) \
@@ -49,10 +52,8 @@ cudaError_t launch_decode(const float*, int64_t, int64_t, int64_t, int64_t, int,
 cudaError_t launch_dec_init(lac_dec_state*, int64_t, int, const uint8_t*, const int64_t*, cudaStream_t);
 // coder_kernels.cu
 cudaError_t launch_enc_init(lac_enc_state*, int64_t, int, cudaStream_t);
-cudaError_t launch_encode_pairs(const uint32_t*, int64_t, int64_t, int64_t, int64_t, const int32_t*, lac_enc_state*,
-                                uint8_t*, int64_t, int, int, cudaStream_t);
-cudaError_t launch_encode_pairs_at(const uint32_t*, int64_t, int64_t, int64_t, int64_t, const int32_t*, int64_t,
-                                   lac_enc_state*, uint8_t*, int64_t, int, int, cudaStream_t);
+cudaError_t launch_encode_pairs(const uint32_t*, int64_t, int64_t, int64_t, int64_t, const int32_t*, int64_t,
+                                lac_enc_state*, uint8_t*, int64_t, int, int, cudaStream_t);
 cudaError_t launch_encode_logits(const float*, int64_t, int64_t, int64_t, int64_t, int, const int32_t*, int64_t,
                                  const int32_t*, lac_enc_state*, uint8_t*, int64_t, int, int, void*, size_t,
                                  cudaStream_t);

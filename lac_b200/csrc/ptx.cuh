@@ -47,13 +47,6 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 __device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void fence_acq_rel_cta() { asm volatile("fence.acq_rel.cta;" ::: "memory"); }
 
-__device__ __forceinline__ float4 ldg_stream4(const float* p) {
-    float4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-                 : "l"(p));
-    return v;
-}
 __device__ __forceinline__ float ldg_stream1(const float* p) {
     float v;
     asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
