@@ -171,8 +171,8 @@ int lac_ac_encode_uniform(const int32_t* d_syms, int64_t n_streams, int64_t T, i
     if ((!d_syms && T > 0) || !d_state || !d_out || n_streams < 0 || T < 0 || out_stride < 1 || n_symbols < 1)
         return fail(LAC_E_ARG, "lac_ac_encode_uniform: bad argument");
     if (!prec_ok(prec, 2)) return fail(LAC_E_ARG, "lac_ac_encode_uniform: prec %d outside [2, 60]", prec);
-    CK(lac::launch_uniform_encode(d_syms, n_streams, T, sym_stride, d_ntok, n_symbols, d_state, d_out, out_stride,
-                                  finish, prec, (cudaStream_t)stream),
+    CK(lac::launch_table_encode(lac::Uniform{n_symbols}, d_syms, sym_stride, n_streams, T, d_ntok, d_state, d_out,
+                                out_stride, finish ? lac::kFlushAc : lac::kFlushNone, prec, (cudaStream_t)stream),
        "lac_ac_encode_uniform");
     return LAC_OK;
 }
@@ -183,8 +183,8 @@ int lac_ac_decode_uniform(int64_t n_streams, int64_t T, const int32_t* d_ntok, i
     if (!d_state || !d_bytes || !d_offsets || (!d_syms && T > 0) || n_streams < 0 || T < 0 || n_symbols < 1)
         return fail(LAC_E_ARG, "lac_ac_decode_uniform: bad argument");
     if (!prec_ok(prec, 2)) return fail(LAC_E_ARG, "lac_ac_decode_uniform: prec %d outside [2, 60]", prec);
-    CK(lac::launch_uniform_decode(n_streams, T, d_ntok, n_symbols, d_state, d_bytes, d_offsets, d_syms, sym_stride,
-                                  prec, (cudaStream_t)stream),
+    CK(lac::launch_table_decode(lac::Uniform{n_symbols}, n_streams, T, d_ntok, d_state, d_bytes, d_offsets, d_syms,
+                                sym_stride, prec, (cudaStream_t)stream),
        "lac_ac_decode_uniform");
     return LAC_OK;
 }
@@ -198,9 +198,9 @@ int lac_ac_encode_tables(const int64_t* d_dist, int32_t vocab, int64_t stream_st
         out_stride < 1)
         return fail(LAC_E_ARG, "lac_ac_encode_tables: bad argument");
     if (!prec_ok(prec, 2)) return fail(LAC_E_ARG, "lac_ac_encode_tables: prec %d outside [2, 60]", prec);
-    CK(lac::launch_ac_tables_encode(d_dist, vocab, stream_stride, tok_stride, d_minp, minp_stream_stride,
-                                    minp_tok_stride, d_syms, sym_stride, n_streams, T, d_ntok, d_state, d_out, out_stride,
-                                    finish, prec, flags, (cudaStream_t)stream),
+    const lac::Cdf m{vocab, d_dist, stream_stride, tok_stride, d_minp, minp_stream_stride, minp_tok_stride, flags};
+    CK(lac::launch_table_encode(m, d_syms, sym_stride, n_streams, T, d_ntok, d_state, d_out, out_stride,
+                                finish ? lac::kFlushAc : lac::kFlushNone, prec, (cudaStream_t)stream),
        "lac_ac_encode_tables");
     return LAC_OK;
 }
@@ -213,9 +213,9 @@ int lac_ac_decode_tables(const int64_t* d_dist, int32_t vocab, int64_t stream_st
     if (!d_dist || !d_minp || !d_state || !d_bytes || !d_offsets || !d_syms || vocab < 1 || n_streams < 0 || T < 0)
         return fail(LAC_E_ARG, "lac_ac_decode_tables: bad argument");
     if (!prec_ok(prec, 2)) return fail(LAC_E_ARG, "lac_ac_decode_tables: prec %d outside [2, 60]", prec);
-    CK(lac::launch_ac_tables_decode(d_dist, vocab, stream_stride, tok_stride, d_minp, minp_stream_stride,
-                                    minp_tok_stride, n_streams, T, d_ntok, d_state, d_bytes, d_offsets, d_syms,
-                                    sym_stride, prec, flags, (cudaStream_t)stream),
+    const lac::Cdf m{vocab, d_dist, stream_stride, tok_stride, d_minp, minp_stream_stride, minp_tok_stride, flags};
+    CK(lac::launch_table_decode(m, n_streams, T, d_ntok, d_state, d_bytes, d_offsets, d_syms, sym_stride, prec,
+                                (cudaStream_t)stream),
        "lac_ac_decode_tables");
     return LAC_OK;
 }
@@ -227,8 +227,10 @@ int lac_acs_encode_tables(const uint64_t* d_cdf, int32_t vocab, int64_t stream_s
     if (!d_cdf || (!d_syms && T > 0) || !d_state || !d_out || vocab < 1 || n_streams < 0 || T < 0 || out_stride < 1)
         return fail(LAC_E_ARG, "lac_acs_encode_tables: bad argument");
     if (!prec_ok(prec, 2)) return fail(LAC_E_ARG, "lac_acs_encode_tables: prec %d outside [2, 60]", prec);
-    CK(lac::launch_acs_tables_encode(d_cdf, vocab, stream_stride, tok_stride, d_syms, sym_stride, n_streams, T, d_ntok,
-                                     d_state, d_out, out_stride, finish, prec, (cudaStream_t)stream),
+    // finish 1: flush_compress (the reference's), 2: the safe termination, anything else: no flush
+    const int flush = finish == 1 ? lac::kFlushCompress : (finish == 2 ? lac::kFlushAc : lac::kFlushNone);
+    CK(lac::launch_table_encode(lac::Acs{vocab, d_cdf, stream_stride, tok_stride}, d_syms, sym_stride, n_streams, T,
+                                d_ntok, d_state, d_out, out_stride, flush, prec, (cudaStream_t)stream),
        "lac_acs_encode_tables");
     return LAC_OK;
 }
@@ -240,8 +242,8 @@ int lac_acs_decode_tables(const uint64_t* d_cdf, int32_t vocab, int64_t stream_s
     if (!d_cdf || !d_state || !d_bytes || !d_offsets || !d_syms || vocab < 1 || n_streams < 0 || T < 0)
         return fail(LAC_E_ARG, "lac_acs_decode_tables: bad argument");
     if (!prec_ok(prec, 2)) return fail(LAC_E_ARG, "lac_acs_decode_tables: prec %d outside [2, 60]", prec);
-    CK(lac::launch_acs_tables_decode(d_cdf, vocab, stream_stride, tok_stride, n_streams, T, d_ntok, d_state, d_bytes,
-                                     d_offsets, d_syms, sym_stride, prec, (cudaStream_t)stream),
+    CK(lac::launch_table_decode(lac::Acs{vocab, d_cdf, stream_stride, tok_stride}, n_streams, T, d_ntok, d_state,
+                                d_bytes, d_offsets, d_syms, sym_stride, prec, (cudaStream_t)stream),
        "lac_acs_decode_tables");
     return LAC_OK;
 }

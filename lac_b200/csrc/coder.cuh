@@ -31,13 +31,13 @@ struct BitWriter {
     int nacc;        // 0..7 between calls
     uint32_t status;
 
-    __device__ void open(uint8_t* o, uint64_t c, uint64_t nb) {
+    __device__ void open(uint8_t* o, uint64_t c, uint64_t nb, uint32_t st) {
         out = o;
         cap = c;
         nbits = nb;
         nacc = (int)(nb & 7);
         acc = 0;
-        status = 0;
+        status = st;
         if (nacc && (nb >> 3) < cap) acc = out[nb >> 3] >> (8 - nacc);
     }
     // add E (signed, |E| < 2^(k+3)) as the next k bits, k <= 40
@@ -276,16 +276,6 @@ __device__ inline void ac_flush(int64_t& l, int64_t& h, int P, Writer& bw) {
     }
     l = 0;
     h = denom - 1;
-}
-
-// ---------------------------------------------------------------- Region pieces (ACSampler)
-// Region.step's interval update (arithmetic_coding.py:160-168): map(v, d) = low + span*v // d.
-__device__ __forceinline__ void acs_narrow(int64_t& low, int64_t& high, uint64_t cl, uint64_t ch, uint64_t den) {
-    u128 span = (u128)(uint64_t)(high - low + 1);
-    int64_t nl = low + (int64_t)(uint64_t)((span * cl) / den);
-    int64_t nh = low + (int64_t)(uint64_t)((span * ch) / den) - 1;
-    low = nl;
-    high = nh;
 }
 
 }  // namespace coder

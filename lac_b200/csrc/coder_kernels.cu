@@ -1,19 +1,11 @@
-// coder_kernels.cu -- batched multi-stream range coder kernels (north-star part (b)).
+// coder_kernels.cu -- batched multi-stream range coder kernels on the logits path (north-star part (b)).
 //
 //   encode_pairs_staged_kernel   one lane per stream, 4 streams per warp; (lo, hi) pairs on the fixed total
 //                         2^32 (output of the lookup) -> MSB-first bytes.  low / high live in registers, the k
 //                         renormalisation bits of a token are appended in one step with carry resolution
 //                         (coder.cuh) into a shared-memory stage that the whole warp flushes.
 //   encode_fused_kernel   symbol ranges + coder in one launch for the model-in-the-loop step (T <= 4)
-//   ac_tables_*           one warp per stream; int64 inclusive cumulative tables exactly as
-//                         CDFPredictor.dist holds them, including fudged_dist
-//                         (arith_code.py:83-93) evaluated as a parallel prefix-max:
-//                           p_i = p_{i-1} + max(1, min(w - p_{i-1} - V + i + 1, f_i - p_{i-1}))
-//                               = max(p_{i-1} + 1, g_i),   g_i = min(w - V + i + 1, f_i)
-//                           =>  p_i - i = max(1, max_{j<=i} (g_j - j))
-//                         which holds for arbitrary f_i (also the wrapped int64 products of
-//                         Llama_AC, flag LAC_F_WRAP64).
-//   acs_tables_*          ACSampler / Region semantics (arithmetic_coding.py).
+// The coders on tables the caller supplies (CDFPredictor, ACSampler, Predictor(n)) are in table_coders.cu.
 #include <cstdint>
 #include <cuda_runtime.h>
 
@@ -22,30 +14,6 @@
 #include "rowsum.cuh"
 
 namespace lac {
-
-using coder::i128;
-using coder::u128;
-
-__device__ __forceinline__ i128 fdiv(i128 a, i128 b) {  // Python floor division, b > 0
-    i128 q = a / b;
-    if ((a % b != 0) && (a < 0)) q -= 1;
-    return q;
-}
-__device__ __forceinline__ i128 cdiv(i128 a, i128 b) { return -fdiv(-a, b); }
-
-__device__ __forceinline__ int64_t warp_max_i64(int64_t v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        int64_t t = __shfl_xor_sync(0xffffffffu, v, o);
-        v = t > v ? t : v;
-    }
-    return v;
-}
-__device__ __forceinline__ int64_t warp_sum_i64(int64_t v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 
 // ------------------------------------------------------------------ pairs encoder
 // One warp per kPairsSpb streams (lanes 0 .. kPairsSpb-1 run A_to_bin, low / high in registers).  The bytes of a
@@ -232,88 +200,6 @@ encode_fused_kernel(const __grid_constant__ EncParams ep) {
     }
 }
 
-// ------------------------------------------------------------------ uniform Predictor(n) (arith_code.py:64-74)
-// The reference's base class maps symbol s of n to [floor(s w / n), floor((s + 1) w / n)) -- floor, not the ceil of
-// CDFPredictor.  AC() without arguments is AC(Predictor(3), 16).  One thread per stream.
-__global__ void uniform_encode_kernel(const int32_t* __restrict__ syms, int64_t n_streams, int64_t T, int64_t sym_stride,
-                                      const int32_t* __restrict__ ntok, int nsym, lac_enc_state* __restrict__ state,
-                                      uint8_t* __restrict__ out, int64_t out_stride, int finish, int P) {
-    int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    int64_t l = state[s].low, h = state[s].high;
-    coder::BitWriter bw;
-    bw.open(out + s * out_stride, (uint64_t)out_stride, state[s].nbits);
-    bw.status = state[s].status;
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
-    for (int64_t t = 0; t < Ts; t++) {
-        const int sym = syms[s * sym_stride + t];
-        if (sym < 0 || sym >= nsym) {
-            bw.status |= LAC_ST_SYMBOL;
-            break;
-        }
-        const u128 w = (u128)(uint64_t)(h - l + 1);
-        const int64_t r0 = (int64_t)(((u128)(uint32_t)sym * w) / (uint32_t)nsym);          // symbol_to_range :69-70
-        const int64_t r1 = (int64_t)((((u128)(uint32_t)sym + 1) * w) / (uint32_t)nsym);
-        if (r1 <= r0) {  // zero-width symbol (w < n): the reference would never terminate
-            bw.status |= LAC_ST_TABLE;
-            break;
-        }
-        h = l + r1 - 1;  // receive_symbol :169-175
-        l += r0;
-        int k = coder::renorm_count((uint64_t)(h - l + 1), P);
-        int64_t E = coder::renorm_apply(l, h, P, k);
-        bw.append(E, k);
-        if (bw.status & LAC_ST_CAP) break;
-    }
-    if (finish && !(bw.status & (LAC_ST_TABLE | LAC_ST_SYMBOL | LAC_ST_CAP))) coder::ac_flush(l, h, P, bw);
-    bw.close();
-    state[s].low = l;
-    state[s].high = h;
-    state[s].nbits = bw.nbits;
-    state[s].status = bw.status;
-}
-
-// Decoder: the symbol whose floor-mapped range holds the code value, i.e. the largest s with
-// floor(s w / n) <= v - l, s = floor(((v - l + 1) n - 1) / w).  (The reference's val_to_symbol, (v n) // w, is not
-// that symbol at range boundaries; its decoder asserts there.  See tests/golden/ac_uniform.npz.)
-__global__ void uniform_decode_kernel(int64_t n_streams, int64_t T, const int32_t* __restrict__ ntok, int nsym,
-                                      lac_dec_state* __restrict__ state, const uint8_t* __restrict__ bytes,
-                                      const int64_t* __restrict__ offsets, int32_t* __restrict__ syms,
-                                      int64_t sym_stride, int P) {
-    int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    int64_t l = state[s].low, h = state[s].high, v = state[s].value;
-    uint64_t pos = state[s].pos;
-    uint32_t status = state[s].status;
-    const uint8_t* data = bytes + offsets[s];
-    const uint64_t nbytes = (uint64_t)(offsets[s + 1] - offsets[s]);
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
-    for (int64_t t = 0; t < Ts; t++) {
-        const u128 w = (u128)(uint64_t)(h - l + 1);
-        const u128 x = (u128)(uint64_t)(v - l);
-        const int64_t sym = (int64_t)(((x + 1) * (uint32_t)nsym - 1) / w);
-        const int64_t r0 = (int64_t)(((u128)(uint64_t)sym * w) / (uint32_t)nsym);
-        const int64_t r1 = (int64_t)((((u128)(uint64_t)sym + 1) * w) / (uint32_t)nsym);
-        if (sym >= nsym || r1 <= r0) {
-            status |= LAC_ST_TABLE;
-            break;
-        }
-        h = l + r1 - 1;
-        l += r0;
-        const int64_t off = v - l;
-        int k = coder::renorm_count((uint64_t)(h - l + 1), P);
-        coder::renorm_apply(l, h, P, k);
-        v = l + (off << k) + (int64_t)coder::read_bits(data, nbytes, pos, k);
-        pos += (uint64_t)k;
-        syms[s * sym_stride + t] = (int32_t)sym;
-    }
-    state[s].low = l;
-    state[s].high = h;
-    state[s].value = v;
-    state[s].pos = pos;
-    state[s].status = status;
-}
-
 __global__ void enc_init_kernel(lac_enc_state* state, int64_t n, int P) {
     int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (s >= n) return;
@@ -322,313 +208,6 @@ __global__ void enc_init_kernel(lac_enc_state* state, int64_t n, int P) {
     state[s].nbits = 0;
     state[s].status = 0;
     state[s]._pad = 0;
-}
-
-// ------------------------------------------------------------------ CDFPredictor on a warp
-struct TableCtx {
-    const int64_t* tbl;
-    int V;
-    int64_t minp;
-    int wrap;
-};
-
-// f_i of fudged_dist: (dist[i] * denom) // dist[-1]   (np.int64-wrapped under LAC_F_WRAP64)
-__device__ __forceinline__ i128 fudge_f(const TableCtx& c, int i, int64_t w, int64_t last) {
-    i128 prod = c.wrap ? (i128)(int64_t)((uint64_t)c.tbl[i] * (uint64_t)w) : (i128)c.tbl[i] * (i128)w;
-    return fdiv(prod, (i128)last);
-}
-__device__ __forceinline__ bool is_fudged(const TableCtx& c, int64_t w, int64_t last) {
-    i128 thr = c.wrap ? (i128)(int64_t)((uint64_t)w * (uint64_t)c.minp) : (i128)w * (i128)c.minp;
-    return !((i128)last <= thr);
-}
-// g_i - i, clamped into int64 (|f| can reach 2^63 / 1 only for degenerate tables)
-__device__ __forceinline__ int64_t fudge_key(const TableCtx& c, int i, int64_t w, int64_t last) {
-    i128 f = fudge_f(c, i, w, last);
-    i128 cap = (i128)w - c.V + i + 1;
-    i128 g = f < cap ? f : cap;
-    g -= i;
-    const i128 lim = ((i128)1) << 62;
-    if (g > lim) g = lim;
-    if (g < -lim) g = -lim;
-    return (int64_t)g;
-}
-
-// Warp-cooperative: the three fudged cumulative values p[a-1] (0 if a == 0), p[a], p[V-1].
-__device__ inline void fudged_three(const TableCtx& c, int a, int64_t w, int64_t last, int lane,
-                                    int64_t& p_lo, int64_t& p_hi, int64_t& p_last) {
-    const int64_t NEG = -(1ll << 62);
-    int64_t m_lo = NEG, m_hi = NEG, m_all = NEG;
-    for (int i = lane; i < c.V; i += 32) {
-        int64_t k = fudge_key(c, i, w, last);
-        if (i < a) m_lo = k > m_lo ? k : m_lo;
-        if (i <= a) m_hi = k > m_hi ? k : m_hi;
-        m_all = k > m_all ? k : m_all;
-    }
-    m_lo = warp_max_i64(m_lo);
-    m_hi = warp_max_i64(m_hi);
-    m_all = warp_max_i64(m_all);
-    p_lo = a > 0 ? (a - 1) + (m_lo > 1 ? m_lo : 1) : 0;
-    p_hi = a + (m_hi > 1 ? m_hi : 1);
-    p_last = (c.V - 1) + (m_all > 1 ? m_all : 1);
-}
-
-// symbol_to_range (arith_code.py:98-110): offsets r0, r1 inside a width-w interval.
-__device__ inline bool table_range(const TableCtx& c, int sym, int64_t w, int lane, int64_t& r0, int64_t& r1) {
-    const int64_t last = c.tbl[c.V - 1];
-    int64_t ld, hd, d;
-    if (is_fudged(c, w, last)) {
-        fudged_three(c, sym, w, last, lane, ld, hd, d);
-    } else {
-        ld = sym > 0 ? c.tbl[sym - 1] : 0;
-        hd = c.tbl[sym];
-        d = last;
-    }
-    if (d <= 0) return false;
-    r0 = (int64_t)cdiv((i128)ld * w, (i128)d);
-    r1 = (int64_t)cdiv((i128)hd * w, (i128)d);
-    return r1 > r0;
-}
-
-// val_to_symbol (arith_code.py:94-97): bisect_right(fudged_dist(w), (x * dist[-1]) // w).
-__device__ inline int table_symbol(const TableCtx& c, int64_t x, int64_t w, int lane) {
-    const int64_t last = c.tbl[c.V - 1];
-    int64_t cnt = 0;
-    if (!is_fudged(c, w, last)) {
-        i128 target = fdiv((i128)x * last, (i128)w);
-        for (int i = lane; i < c.V; i += 32) cnt += ((i128)c.tbl[i] <= target);
-        return (int)warp_sum_i64(cnt);
-    }
-    // fudged: lane owns the contiguous block [b, e); running max of (g_j - j) carried across lanes
-    const int64_t NEG = -(1ll << 62);
-    const int per = (c.V + 31) / 32;
-    const int b = lane * per < c.V ? lane * per : c.V, e = b + per < c.V ? b + per : c.V;
-    int64_t m = NEG;
-    for (int i = b; i < e; i++) {
-        int64_t k = fudge_key(c, i, w, last);
-        m = k > m ? k : m;
-    }
-    int64_t inc = m;  // inclusive max-scan over lanes
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        int64_t t = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc = t > inc ? t : inc;
-    }
-    int64_t m_all = __shfl_sync(0xffffffffu, inc, 31);
-    int64_t run = __shfl_up_sync(0xffffffffu, inc, 1);
-    if (lane == 0) run = NEG;
-    const int64_t d = (c.V - 1) + (m_all > 1 ? m_all : 1);
-    const i128 target = fdiv((i128)x * d, (i128)w);
-    for (int i = b; i < e; i++) {
-        int64_t k = fudge_key(c, i, w, last);
-        run = k > run ? k : run;
-        int64_t p = i + (run > 1 ? run : 1);
-        cnt += ((i128)p <= target);
-    }
-    return (int)warp_sum_i64(cnt);
-}
-
-__device__ __forceinline__ TableCtx table_ctx(const int64_t* dist, int V, int64_t ss, int64_t ts,
-                                              const int64_t* minp, int64_t mss, int64_t mts, int64_t s,
-                                              int64_t t, int flags) {
-    TableCtx c;
-    c.tbl = dist + s * ss + t * ts;
-    c.V = V;
-    c.minp = minp[s * mss + t * mts];
-    c.wrap = (flags & LAC_F_WRAP64) != 0;
-    return c;
-}
-
-// ------------------------------------------------------------------ A_to_bin on tables
-__global__ void ac_tables_encode_kernel(const int64_t* __restrict__ dist, int V, int64_t ss, int64_t ts,
-                                        const int64_t* __restrict__ minp, int64_t mss, int64_t mts,
-                                        const int32_t* __restrict__ syms, int64_t sym_stride, int64_t n_streams,
-                                        int64_t T, const int32_t* __restrict__ ntok,
-                                        lac_enc_state* __restrict__ state, uint8_t* __restrict__ out,
-                                        int64_t out_stride, int finish, int P, int flags) {
-    const int lane = threadIdx.x & 31;
-    int64_t s = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-    if (s >= n_streams) return;
-    int64_t l = state[s].low, h = state[s].high;
-    coder::BitWriter bw;
-    bw.open(out + s * out_stride, (uint64_t)out_stride, state[s].nbits);
-    bw.status = state[s].status;
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
-    for (int64_t t = 0; t < Ts; t++) {
-        const int sym = syms[s * sym_stride + t];
-        if (sym < 0 || sym >= V) {
-            bw.status |= LAC_ST_SYMBOL;
-            break;
-        }
-        TableCtx c = table_ctx(dist, V, ss, ts, minp, mss, mts, s, t, flags);
-        int64_t r0, r1;
-        if (!table_range(c, sym, h - l + 1, lane, r0, r1)) {
-            bw.status |= LAC_ST_TABLE;
-            break;
-        }
-        h = l + r1 - 1;
-        l += r0;
-        int k = coder::renorm_count((uint64_t)(h - l + 1), P);
-        int64_t E = coder::renorm_apply(l, h, P, k);
-        if (lane == 0) bw.append(E, k);
-        if (__shfl_sync(0xffffffffu, bw.status, 0) & LAC_ST_CAP) break;
-    }
-    if (lane == 0) {
-        if (finish && !(bw.status & (LAC_ST_TABLE | LAC_ST_SYMBOL | LAC_ST_CAP))) coder::ac_flush(l, h, P, bw);
-        bw.close();
-        state[s].low = l;
-        state[s].high = h;
-        state[s].nbits = bw.nbits;
-        state[s].status = bw.status;
-    }
-}
-
-__global__ void ac_tables_decode_kernel(const int64_t* __restrict__ dist, int V, int64_t ss, int64_t ts,
-                                        const int64_t* __restrict__ minp, int64_t mss, int64_t mts,
-                                        int64_t n_streams, int64_t T, const int32_t* __restrict__ ntok,
-                                        lac_dec_state* __restrict__ state, const uint8_t* __restrict__ bytes,
-                                        const int64_t* __restrict__ offsets, int32_t* __restrict__ syms,
-                                        int64_t sym_stride, int P, int flags) {
-    const int lane = threadIdx.x & 31;
-    int64_t s = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-    if (s >= n_streams) return;
-    int64_t l = state[s].low, h = state[s].high, v = state[s].value;
-    uint64_t pos = state[s].pos;
-    uint32_t status = state[s].status;
-    const uint8_t* data = bytes + offsets[s];
-    const uint64_t nbytes = (uint64_t)(offsets[s + 1] - offsets[s]);
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
-    for (int64_t t = 0; t < Ts; t++) {
-        TableCtx c = table_ctx(dist, V, ss, ts, minp, mss, mts, s, t, flags);
-        const int64_t w = h - l + 1;
-        int sym = table_symbol(c, v - l, w, lane);
-        int64_t r0, r1;
-        if (sym >= V || !table_range(c, sym, w, lane, r0, r1)) {
-            status |= LAC_ST_TABLE;
-            break;
-        }
-        h = l + r1 - 1;
-        l += r0;
-        const int64_t off = v - l;
-        int k = coder::renorm_count((uint64_t)(h - l + 1), P);
-        coder::renorm_apply(l, h, P, k);
-        v = l + (off << k) + (int64_t)coder::read_bits(data, nbytes, pos, k);
-        pos += (uint64_t)k;
-        if (lane == 0) syms[s * sym_stride + t] = sym;
-    }
-    if (lane == 0) {
-        state[s].low = l;
-        state[s].high = h;
-        state[s].value = v;
-        state[s].pos = pos;
-        state[s].status = status;
-    }
-}
-
-// ------------------------------------------------------------------ ACSampler on tables
-__global__ void acs_tables_encode_kernel(const uint64_t* __restrict__ cdf, int V, int64_t ss, int64_t ts,
-                                         const int32_t* __restrict__ syms, int64_t sym_stride, int64_t n_streams,
-                                         int64_t T, const int32_t* __restrict__ ntok,
-                                         lac_enc_state* __restrict__ state, uint8_t* __restrict__ out,
-                                         int64_t out_stride, int finish, int P) {
-    int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    int64_t low = state[s].low, high = state[s].high;
-    coder::BitWriter bw;
-    bw.open(out + s * out_stride, (uint64_t)out_stride, state[s].nbits);
-    bw.status = state[s].status;
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
-    for (int64_t t = 0; t < Ts; t++) {
-        const int tok = syms[s * sym_stride + t];
-        if (tok < 0 || tok >= V) {
-            bw.status |= LAC_ST_SYMBOL;
-            break;
-        }
-        const uint64_t* c = cdf + s * ss + t * ts;
-        // sample_scaled_cdf compress path, arithmetic_coding.py:85-87
-        uint64_t cl = tok ? c[tok - 1] : 0, ch = c[tok], den = c[V - 1];
-        if (den == 0 || ch <= cl) {
-            bw.status |= LAC_ST_TABLE;
-            break;
-        }
-        coder::acs_narrow(low, high, cl, ch, den);
-        if (high < low) {
-            bw.status |= LAC_ST_TABLE;
-            break;
-        }
-        int k = coder::renorm_count((uint64_t)(high - low + 1), P);
-        bw.append(coder::renorm_apply(low, high, P, k), k);
-        if (bw.status & LAC_ST_CAP) break;
-    }
-    if (finish == 1 && !(bw.status & (LAC_ST_TABLE | LAC_ST_SYMBOL | LAC_ST_CAP))) {
-        // flush_compress, arithmetic_coding.py:50-56: step(1, 2, 3), drain the carry buffer, reset.
-        // Bit-exact with the reference, but the bits do not pin the final region (DESIGN.md
-        // section 6): the last tokens may be undecodable by ANY decoder.
-        coder::acs_narrow(low, high, 1, 2, 3);
-        int k = coder::renorm_count((uint64_t)(high - low + 1), P);
-        bw.append(coder::renorm_apply(low, high, P, k), k);
-        low = 0;
-        high = (1ll << P) - 1;
-    } else if (finish == 2 && !(bw.status & (LAC_ST_TABLE | LAC_ST_SYMBOL | LAC_ST_CAP))) {
-        // safe termination: shortest bit string whose every continuation stays inside [low, high]
-        // (A_to_bin.flush, arith_code.py:193-202) -- always decodable
-        coder::ac_flush(low, high, P, bw);
-    }
-    bw.close();
-    state[s].low = low;
-    state[s].high = high;
-    state[s].nbits = bw.nbits;
-    state[s].status = bw.status;
-}
-
-// Decoder for ACSampler streams: symbol whose encoder interval [map(c[i-1]), map(c[i]) - 1]
-// contains the value; map(c) <= v  <=>  c <= ceil((v - low + 1) * den / span) - 1.
-__global__ void acs_tables_decode_kernel(const uint64_t* __restrict__ cdf, int V, int64_t ss, int64_t ts,
-                                         int64_t n_streams, int64_t T, const int32_t* __restrict__ ntok,
-                                         lac_dec_state* __restrict__ state, const uint8_t* __restrict__ bytes,
-                                         const int64_t* __restrict__ offsets, int32_t* __restrict__ syms,
-                                         int64_t sym_stride, int P) {
-    const int lane = threadIdx.x & 31;
-    int64_t s = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-    if (s >= n_streams) return;
-    int64_t low = state[s].low, high = state[s].high, v = state[s].value;
-    uint64_t pos = state[s].pos;
-    uint32_t status = state[s].status;
-    const uint8_t* data = bytes + offsets[s];
-    const uint64_t nbytes = (uint64_t)(offsets[s + 1] - offsets[s]);
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
-    for (int64_t t = 0; t < Ts; t++) {
-        const uint64_t* c = cdf + s * ss + t * ts;
-        const uint64_t den = c[V - 1];
-        const u128 span = (u128)(uint64_t)(high - low + 1);
-        if (den == 0) {
-            status |= LAC_ST_TABLE;
-            break;
-        }
-        const u128 num = (u128)(uint64_t)(v - low + 1) * den;
-        const u128 tau = (num + span - 1) / span - 1;
-        int64_t cnt = 0;
-        for (int i = lane; i < V; i += 32) cnt += ((u128)c[i] <= tau);
-        const int tok = (int)warp_sum_i64(cnt);
-        if (tok >= V) {
-            status |= LAC_ST_TABLE;
-            break;
-        }
-        uint64_t cl = tok ? c[tok - 1] : 0, ch = c[tok];
-        coder::acs_narrow(low, high, cl, ch, den);
-        const int64_t off = v - low;
-        int k = coder::renorm_count((uint64_t)(high - low + 1), P);
-        coder::renorm_apply(low, high, P, k);
-        v = low + (off << k) + (int64_t)coder::read_bits(data, nbytes, pos, k);
-        pos += (uint64_t)k;
-        if (lane == 0) syms[s * sym_stride + t] = tok;
-    }
-    if (lane == 0) {
-        state[s].low = low;
-        state[s].high = high;
-        state[s].value = v;
-        state[s].pos = pos;
-        state[s].status = status;
-    }
 }
 
 // ------------------------------------------------------------------ status collection
@@ -734,65 +313,6 @@ cudaError_t launch_encode_logits(const float* logits, int64_t n, int64_t T, int6
     }
     const cudaError_t ef = scratch_put(&sc, st);
     return e != cudaSuccess ? e : ef;
-}
-
-cudaError_t launch_uniform_encode(const int32_t* syms, int64_t n, int64_t T, int64_t sym_stride, const int32_t* ntok,
-                                  int nsym, lac_enc_state* state, uint8_t* out, int64_t out_stride, int finish, int P,
-                                  cudaStream_t st) {
-    if (n == 0) return cudaSuccess;
-    uniform_encode_kernel<<<(unsigned)((n + 31) / 32), 32, 0, st>>>(syms, n, T, sym_stride, ntok, nsym, state, out,
-                                                                    out_stride, finish, P);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_uniform_decode(int64_t n, int64_t T, const int32_t* ntok, int nsym, lac_dec_state* state,
-                                  const uint8_t* bytes, const int64_t* offsets, int32_t* syms, int64_t sym_stride,
-                                  int P, cudaStream_t st) {
-    if (n == 0 || T == 0) return cudaSuccess;
-    uniform_decode_kernel<<<(unsigned)((n + 31) / 32), 32, 0, st>>>(n, T, ntok, nsym, state, bytes, offsets, syms,
-                                                                    sym_stride, P);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_ac_tables_encode(const int64_t* dist, int V, int64_t ss, int64_t ts, const int64_t* minp,
-                                    int64_t mss, int64_t mts, const int32_t* syms, int64_t sym_stride, int64_t n,
-                                    int64_t T, const int32_t* ntok, lac_enc_state* state, uint8_t* out,
-                                    int64_t out_stride, int finish, int P, int flags, cudaStream_t st) {
-    if (n == 0) return cudaSuccess;
-    ac_tables_encode_kernel<<<(unsigned)((n + 3) / 4), 128, 0, st>>>(dist, V, ss, ts, minp, mss, mts, syms, sym_stride, n,
-                                                                    T, ntok, state, out, out_stride, finish, P, flags);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_ac_tables_decode(const int64_t* dist, int V, int64_t ss, int64_t ts, const int64_t* minp,
-                                    int64_t mss, int64_t mts, int64_t n, int64_t T, const int32_t* ntok,
-                                    lac_dec_state* state, const uint8_t* bytes, const int64_t* offsets,
-                                    int32_t* syms, int64_t sym_stride, int P, int flags, cudaStream_t st) {
-    if (n == 0) return cudaSuccess;
-    ac_tables_decode_kernel<<<(unsigned)((n + 3) / 4), 128, 0, st>>>(dist, V, ss, ts, minp, mss, mts, n, T, ntok,
-                                                                    state, bytes, offsets, syms, sym_stride, P,
-                                                                    flags);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_acs_tables_encode(const uint64_t* cdf, int V, int64_t ss, int64_t ts, const int32_t* syms,
-                                     int64_t sym_stride, int64_t n, int64_t T, const int32_t* ntok,
-                                     lac_enc_state* state, uint8_t* out, int64_t out_stride, int finish, int P,
-                                     cudaStream_t st) {
-    if (n == 0) return cudaSuccess;
-    acs_tables_encode_kernel<<<(unsigned)((n + 31) / 32), 32, 0, st>>>(cdf, V, ss, ts, syms, sym_stride, n, T, ntok,
-                                                                      state, out, out_stride, finish, P);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_acs_tables_decode(const uint64_t* cdf, int V, int64_t ss, int64_t ts, int64_t n, int64_t T,
-                                     const int32_t* ntok, lac_dec_state* state, const uint8_t* bytes,
-                                     const int64_t* offsets, int32_t* syms, int64_t sym_stride, int P,
-                                     cudaStream_t st) {
-    if (n == 0) return cudaSuccess;
-    acs_tables_decode_kernel<<<(unsigned)((n + 3) / 4), 128, 0, st>>>(cdf, V, ss, ts, n, T, ntok, state, bytes,
-                                                                     offsets, syms, sym_stride, P);
-    return cudaGetLastError();
 }
 
 }  // namespace lac

@@ -57,21 +57,36 @@ cudaError_t launch_encode_pairs(const uint32_t*, int64_t, int64_t, int64_t, int6
 cudaError_t launch_encode_logits(const float*, int64_t, int64_t, int64_t, int64_t, int, const int32_t*, int64_t,
                                  const int32_t*, lac_enc_state*, uint8_t*, int64_t, int, int, void*, size_t,
                                  cudaStream_t);
-cudaError_t launch_uniform_encode(const int32_t*, int64_t, int64_t, int64_t, const int32_t*, int, lac_enc_state*,
-                                  uint8_t*, int64_t, int, int, cudaStream_t);
-cudaError_t launch_uniform_decode(int64_t, int64_t, const int32_t*, int, lac_dec_state*, const uint8_t*,
-                                  const int64_t*, int32_t*, int64_t, int, cudaStream_t);
-cudaError_t launch_ac_tables_encode(const int64_t*, int, int64_t, int64_t, const int64_t*, int64_t, int64_t,
-                                    const int32_t*, int64_t, int64_t, int64_t, const int32_t*, lac_enc_state*,
-                                    uint8_t*, int64_t, int, int, int, cudaStream_t);
-cudaError_t launch_ac_tables_decode(const int64_t*, int, int64_t, int64_t, const int64_t*, int64_t, int64_t, int64_t,
-                                    int64_t, const int32_t*, lac_dec_state*, const uint8_t*, const int64_t*,
-                                    int32_t*, int64_t, int, int, cudaStream_t);
-cudaError_t launch_acs_tables_encode(const uint64_t*, int, int64_t, int64_t, const int32_t*, int64_t, int64_t,
-                                     int64_t, const int32_t*, lac_enc_state*, uint8_t*, int64_t, int, int,
-                                     cudaStream_t);
-cudaError_t launch_acs_tables_decode(const uint64_t*, int, int64_t, int64_t, int64_t, int64_t, const int32_t*,
-                                     lac_dec_state*, const uint8_t*, const int64_t*, int32_t*, int64_t, int,
-                                     cudaStream_t);
+
+// table_coders.cu: the table models, symbols [0, n_symbols), and how many threads code one stream (1 or 32)
+struct Uniform {  // Predictor(n)
+    static constexpr int kEncLanes = 1, kDecLanes = 1;
+    int n_symbols;
+};
+struct Cdf {  // CDFPredictor: table (s, t) at dist + s * ss + t * ts, its minp at minp[s * mss + t * mts]
+    static constexpr int kEncLanes = 32, kDecLanes = 32;
+    int n_symbols;
+    const int64_t* dist;
+    int64_t ss, ts;
+    const int64_t* minp;
+    int64_t mss, mts;
+    int flags;
+};
+struct Acs {  // ACSampler: table (s, t) at cdf + s * ss + t * ts
+    static constexpr int kEncLanes = 1, kDecLanes = 32;
+    int n_symbols;
+    const uint64_t* cdf;
+    int64_t ss, ts;
+};
+// how an encode call ends a stream: A_to_bin.flush (coder::ac_flush) or ACSampler's flush_compress
+enum TableFlush { kFlushNone, kFlushAc, kFlushCompress };
+template <class Model>
+cudaError_t launch_table_encode(const Model&, const int32_t* syms, int64_t sym_stride, int64_t n, int64_t T,
+                                const int32_t* ntok, lac_enc_state*, uint8_t* out, int64_t out_stride, int flush,
+                                int P, cudaStream_t);
+template <class Model>
+cudaError_t launch_table_decode(const Model&, int64_t n, int64_t T, const int32_t* ntok, lac_dec_state*,
+                                const uint8_t* bytes, const int64_t* offsets, int32_t* syms, int64_t sym_stride,
+                                int P, cudaStream_t);
 
 }  // namespace lac

@@ -386,21 +386,72 @@ def test_uniform_random(n):
         run_uniform_case(rng, n, prec, S, T, ntok, bad)
 
 
+@pytest.mark.parametrize("n, prec", [(5, 2), (20, 4), (600, 9), (70000, 16), (2 ** 31 - 1, 30)])
+def test_uniform_zero_width_symbols_stop_their_stream(n, prec):
+    """Alphabets wider than the range (n > 2^prec) have symbols whose floor-mapped range is empty, from the first
+    token on.  Such a symbol sets LAC_ST_TABLE and stops its stream before it, unflushed, where the exact reference
+    would loop forever.  Every stream's bytes, bit count and status equal the exact reference's, a stopped stream
+    keeps the coder state from before that symbol, and the streams that code through decode back."""
+    rng = np.random.default_rng(n)
+    L, st = _ffi.lib(), torch.cuda.current_stream().cuda_stream
+    S, T = 37, 8
+    syms = np.full((S, T + 2), 0x7FFF0000, dtype=np.int32)
+    syms[:, :T] = rng.integers(0, n, (S, T))
+    w = 1 << prec
+    syms[0, 0] = next(a for a in range(n) if a * w // n == (a + 1) * w // n)
+    ntok = rng.integers(0, T + 1, S).astype(np.int32)
+    ntok[0] = T
+    d_syms, d_ntok = _dev(syms), _dev(ntok)
+    cap = (T + 3) * (prec + 2) // 8 + 16
+    B = Buffers(S, T, cap)
+    _ffi.check(L.lac_enc_init(B.enc_ptr(), S, prec, st))
+    _ffi.check(L.lac_ac_encode_uniform(d_syms.data_ptr(), S, T, T + 2, d_ntok.data_ptr(), n, B.enc_ptr(), B.out_ptr(),
+                                       cap, 0, prec, st))
+    _ffi.check(L.lac_ac_encode_uniform(None, S, 0, 0, None, n, B.enc_ptr(), B.out_ptr(), cap, 1, prec, st))
+    got, nbits, status = B.streams()
+    state = _state_words(B.enc, S, 4)
+    for s in range(S):
+        enc, want = pyref.A_to_bin(prec), 0
+        try:
+            for a in syms[s, :int(ntok[s])]:
+                enc.receive_symbol(pyref.Predictor(n), int(a))
+            enc.flush()
+        except ZeroDivisionError:
+            want = _ffi.LAC_ST_TABLE
+            assert (state[s, 0], state[s, 1]) == (enc.l, enc.h), (n, prec, s)
+        bits = np.array(enc.out.bits(), dtype=np.uint8)
+        assert status[s] == want and got[s] == _packed(bits) and int(nbits[s]) == len(bits), (n, prec, s, status[s])
+    assert status[0] == _ffi.LAC_ST_TABLE and (status[ntok > 0] == 0).any()
+    dntok = np.where(status == 0, ntok, 0).astype(np.int32)
+    data, offs = B.decoder_input([got[s] if status[s] == 0 else b"" for s in range(S)])
+    _ffi.check(L.lac_dec_init(B.dec[1:].data_ptr(), S, prec, data, offs, st))
+    _ffi.check(L.lac_ac_decode_uniform(S, T, _dev(dntok).data_ptr(), n, B.dec[1:].data_ptr(), data, offs,
+                                       B.back[1:].data_ptr(), B.sym_stride, prec, st))
+    back, dstatus = B.decoded(dntok)
+    for s in range(S):
+        assert np.array_equal(back[s, :int(dntok[s])], syms[s, :int(dntok[s])]) and dstatus[s] == 0, (n, prec, s)
+
+
 # ------------------------------------------------------------------------------------------------ ACSampler
+def acs_row(rng, V, prec):
+    return ref_quant.acs_cdf(rng.dirichlet(np.full(V, float(rng.choice([0.05, 0.5, 2.0])))),
+                             precision=prec).view(np.int64)
+
+
+def acs_symbol(rng, c):
+    """A symbol that keeps a non-empty region at every width: frequency >= 3 on a total ~2^prec."""
+    f = np.diff(np.concatenate([[0], c.astype(object)]))
+    return int(rng.choice(np.nonzero(f >= 3)[0]))
+
+
 def run_acs_case(rng, V, prec, S, T, layout, finish, ntok, bad=None):
     L, st = _ffi.lib(), torch.cuda.current_stream().cuda_stream
     kind, ss, ts, _, _ = layout
-
-    def row():
-        return ref_quant.acs_cdf(rng.dirichlet(np.full(V, float(rng.choice([0.05, 0.5, 2.0])))), precision=prec)
-
-    flat, rows = fill_tables(rng, S, T, V, layout, lambda: row().view(np.int64), JUNK)
+    flat, rows = fill_tables(rng, S, T, V, layout, lambda: acs_row(rng, V, prec), JUNK)
     syms = np.full((S, T + 2), 0x7FFF0000, dtype=np.int32)
     for s in range(S):
-        for t in range(T):  # symbols that keep a non-empty region at every width: frequency >= 3 on a total ~2^prec
-            c = table_of(rows, layout, s, t).astype(object)
-            f = np.diff(np.concatenate([[0], c]))
-            syms[s, t] = int(rng.choice(np.nonzero(f >= 3)[0]))
+        for t in range(T):
+            syms[s, t] = acs_symbol(rng, table_of(rows, layout, s, t))
     for s, v in (bad or {}).items():
         syms[s, 0] = v
     count(f"acs_finish{finish}", V, prec, kind)
@@ -458,3 +509,122 @@ def test_acs_tables_random(seed, finish):
         ntok = rng.integers(0, T + 1, S).astype(np.int32) if rng.random() < 0.6 else np.full(S, T, dtype=np.int32)
         bad = {int(rng.integers(0, S)): int(rng.choice([V, -1]))} if rng.random() < 0.3 else None
         run_acs_case(rng, V, prec, S, T, layout, finish, ntok, bad)
+
+
+def _acs_encode(S, T, V, ss, ts, d_cdf, d_syms, B, finish, prec):
+    """One encode call over all T tokens, then a flush-only call with `finish`."""
+    L, st = _ffi.lib(), torch.cuda.current_stream().cuda_stream
+    _ffi.check(L.lac_enc_init(B.enc_ptr(), S, prec, st))
+    _ffi.check(L.lac_acs_encode_tables(d_cdf.data_ptr(), V, ss, ts, d_syms.data_ptr(), T + 2, S, T, None, B.enc_ptr(),
+                                       B.out_ptr(), B.cap, 0, prec, st))
+    _ffi.check(L.lac_acs_encode_tables(d_cdf.data_ptr(), V, ss, ts, None, 0, S, 0, None, B.enc_ptr(), B.out_ptr(),
+                                       B.cap, finish, prec, st))
+    return B.streams()
+
+
+@pytest.mark.parametrize("finish", [1, 2])
+def test_acs_degenerate_tokens_stop_their_stream(finish):
+    """ACSampler encoder: a zero-frequency token (ch == cl), a token of positive frequency whose sub-interval is empty
+    at the current width (floor(span ch / den) == floor(span cl / den)) and an all-zero table (den == 0) each set
+    LAC_ST_TABLE on their own stream before any bit of that token; the other streams stay bit-exact."""
+    rng = np.random.default_rng(60 + finish)
+    V, prec, S, T = 40, 20, 9, 5
+    ss, ts = T * V + 3, V
+    flat, rows = fill_tables(rng, S, T, V, ("streams", ss, ts, 0, 0), lambda: acs_row(rng, V, prec), JUNK)
+    syms = np.full((S, T + 2), 0x7FFF0000, dtype=np.int32)
+    for (s, t), r in rows.items():
+        syms[s, t] = acs_symbol(rng, r)
+    span = 1 << prec  # every stream's width at its first token
+    zero = np.full(V, 3 * (span // V), dtype=np.int64)
+    zero[7] = 0
+    empty = np.cumsum(np.concatenate([[16 * span], np.ones(V - 1, dtype=np.int64)]))  # frequency-1 tokens, den ~ 16 span
+    den = int(empty[-1])
+    j = next(i for i in range(1, V) if span * int(empty[i]) // den == span * int(empty[i - 1]) // den)
+    bad = {2: (np.cumsum(zero), 7), 4: (empty, j), 6: (np.zeros(V, dtype=np.int64), 0)}
+    for s, (r, tok) in bad.items():
+        flat[s * ss: s * ss + V] = r
+        rows[(s, 0)] = r
+        syms[s, 0] = tok
+    B = Buffers(S, T, (T + 3) * (prec + 2) // 8 + 16)
+    got, nbits, status = _acs_encode(S, T, V, ss, ts, _dev(flat), _dev(syms), B, finish, prec)
+    for s in range(S):
+        try:
+            bits = pyref.acs_encode([rows[(s, t)].view(np.uint64).tolist() for t in range(T)], syms[s, :T].tolist(),
+                                    prec, finish=finish)
+            want = 0
+        except ZeroDivisionError:
+            bits, want = [], _ffi.LAC_ST_TABLE
+        bits = np.array(bits, dtype=np.uint8)
+        assert status[s] == want and got[s] == _packed(bits) and int(nbits[s]) == len(bits), (finish, s, status[s])
+    assert sorted(np.nonzero(status)[0].tolist()) == sorted(bad)
+
+
+def test_acs_finish_other_than_1_or_2_flushes_nothing():
+    """finish 1 is flush_compress and 2 the safe termination; any other value, 3 here, leaves the same bytes and coder
+    state as 0: the unflushed bits of the exact reference."""
+    rng = np.random.default_rng(3)
+    V, prec, S, T = 33, 30, 9, 6
+    flat, rows = fill_tables(rng, S, T, V, ("single", 0, 0, 0, 0), lambda: acs_row(rng, V, prec), JUNK)
+    syms = np.full((S, T + 2), 0x7FFF0000, dtype=np.int32)
+    syms[:, :T] = [[acs_symbol(rng, rows[(0, 0)]) for _ in range(T)] for _ in range(S)]
+    d_cdf, d_syms = _dev(flat), _dev(syms)
+    after = []
+    for finish in (0, 3):
+        B = Buffers(S, T, (T + 3) * (prec + 2) // 8 + 16)
+        got, nbits, status = _acs_encode(S, T, V, 0, 0, d_cdf, d_syms, B, finish, prec)
+        for s in range(S):
+            bits = np.array(pyref.acs_encode([rows[(0, 0)].view(np.uint64).tolist()] * T, syms[s, :T].tolist(), prec,
+                                             finish=0), dtype=np.uint8)
+            assert status[s] == 0 and got[s] == _packed(bits) and int(nbits[s]) == len(bits), (finish, s)
+        after.append((B.out.cpu().numpy(), B.enc.cpu().numpy()))
+    assert np.array_equal(after[0][0], after[1][0]) and np.array_equal(after[0][1], after[1][1])
+
+
+@pytest.mark.parametrize("coder", ["cdf", "acs"])
+def test_table_decoders_flag_an_all_zero_table(coder):
+    """CDFPredictor and ACSampler decoders: an all-zero table at a stream's first token sets LAC_ST_TABLE in that
+    stream's decoder status and writes no symbol; the other streams decode back."""
+    rng = np.random.default_rng(5 if coder == "cdf" else 6)
+    L, st = _ffi.lib(), torch.cuda.current_stream().cuda_stream
+    V, prec, S, T, dead = 50, 40, 7, 4, 3
+    ss, ts = T * V + 3, V
+    if coder == "cdf":
+        flat, rows = fill_tables(rng, S, T, V, ("streams", ss, ts, 0, 0),
+                                 lambda: np.cumsum(random_freqs(rng, V, 30, 0.2)), JUNK)
+    else:
+        flat, rows = fill_tables(rng, S, T, V, ("streams", ss, ts, 0, 0), lambda: acs_row(rng, V, prec), JUNK)
+    syms = np.zeros((S, T), dtype=np.int32)
+    for (s, t), r in rows.items():
+        syms[s, t] = acs_symbol(rng, r) if coder == "acs" else int(rng.choice(np.nonzero(np.diff(r, prepend=0))[0]))
+    flat[dead * ss: dead * ss + V] = 0
+    streams = []
+    for s in range(S):
+        tabs = np.stack([rows[(s, t)] for t in range(T)])
+        if s == dead:
+            streams.append(b"")
+        elif coder == "cdf":
+            streams.append(_packed(orc.ac_encode(tabs, syms[s], prec=prec, stop=1)))
+        else:
+            bits = pyref.acs_encode([r.view(np.uint64).tolist() for r in tabs], syms[s].tolist(), prec, finish=2)
+            streams.append(_packed(np.array(bits, dtype=np.uint8)))
+    # minp of every table at s * T + t; the all-zero table has no positive entry, any minp >= 0 leaves it unfudged
+    minp = np.array([pyref.cdf_minp(rows[(s, t)].tolist()) if s != dead or t else 1
+                     for s in range(S) for t in range(T)], dtype=np.int64)
+    B = Buffers(S, T, 16)
+    data, offs = B.decoder_input(streams)
+    d_cdf, d_minp = _dev(flat), _dev(minp)
+    _ffi.check(L.lac_dec_init(B.dec[1:].data_ptr(), S, prec, data, offs, st))
+    if coder == "cdf":
+        _ffi.check(L.lac_ac_decode_tables(d_cdf.data_ptr(), V, ss, ts, d_minp.data_ptr(), T, 1, S, T, None,
+                                          B.dec[1:].data_ptr(), data, offs, B.back[1:].data_ptr(), B.sym_stride, prec, 0,
+                                          st))
+    else:
+        _ffi.check(L.lac_acs_decode_tables(d_cdf.data_ptr(), V, ss, ts, S, T, None, B.dec[1:].data_ptr(), data, offs,
+                                           B.back[1:].data_ptr(), B.sym_stride, prec, st))
+    dntok = np.full(S, T, dtype=np.int32)
+    dntok[dead] = 0
+    back, dstatus = B.decoded(dntok)
+    assert dstatus[dead] == _ffi.LAC_ST_TABLE, (coder, dstatus)
+    for s in range(S):
+        if s != dead:
+            assert np.array_equal(back[s, :T], syms[s]) and dstatus[s] == 0, (coder, s)
