@@ -22,6 +22,8 @@
  *   arithmetic_coding.py:73-93,50-56,128-208,212-225 ACSampler compress path, flush_compress, Region, CarryBuffer,
  *                                                  packbits          -> lac_acs_encode_tables
  *   arithmetic_coding.py:94-124 ACSampler expand path               -> lac_acs_decode_tables
+ *   arith_code.py:111-135     ProbPredictor with prob(s) = count of s -> lac_ac_encode_adaptive / lac_ac_decode_adaptive
+ *                             (same counts under ACSampler)           -> lac_acs_encode_adaptive / lac_acs_decode_adaptive
  *
  * Workspace: the logits-driven calls need 256 * ceil(vocab / 32768) bytes of device scratch per logits row they
  * look at in one launch (lac_workspace_bytes).  Pass d_ws / ws_bytes to keep the call free of allocations (what a
@@ -39,7 +41,7 @@
 extern "C" {
 #endif
 
-#define LAC_ABI_VERSION 2
+#define LAC_ABI_VERSION 3
 
 typedef enum {
     LAC_OK = 0,
@@ -212,6 +214,36 @@ int lac_acs_decode_tables(const uint64_t *d_cdf, int32_t vocab, int64_t stream_s
                           int64_t n_streams, int64_t T, const int32_t *d_ntok, lac_dec_state *d_state,
                           const uint8_t *d_bytes, const int64_t *d_offsets, int32_t *d_syms,
                           int64_t sym_stride, int prec, void *stream);
+
+/* ------------------------------------------------------------------------------------
+ * Adaptive frequency models: prob(s) = counts[s], and after every coded or decoded token
+ * counts[sym] += inc (the reference predictor reads its table, then accepts the symbol).
+ * The counts live on the device: int64 [n_streams][vocab], stream s at d_counts + s * vocab,
+ * read at entry and written back at exit, so a stream can be fed in several calls.  Encoder and
+ * decoder each need their own copy, starting from the same counts.
+ *   lac_ac_*:  CDFPredictor semantics on dist = inclusive cumsum(counts), minp = the smallest
+ *              positive count, fudged_dist when dist[-1] > w * minp (arith_code.py:83-135).
+ *   lac_acs_*: ACSampler semantics on cdf = cumsum(counts); finish as lac_acs_encode_tables.
+ * Bounds: 1 <= vocab <= LAC_ADAPTIVE_MAX_VOCAB, inc >= 0 (0: a static table).  A stream stops
+ * with LAC_ST_TABLE, the others going on, on a negative count, a table total that would reach
+ * 2^62, a symbol of zero width or a zero total; LAC_ST_SYMBOL on a symbol outside [0, vocab).
+ * Counts advance for exactly the tokens that narrowed the interval, so a stopped stream's state
+ * and counts stay a consistent pair.  Everything else as for the table coders.
+ * ---------------------------------------------------------------------------------- */
+#define LAC_ADAPTIVE_MAX_VOCAB 4096
+
+int lac_ac_encode_adaptive(int64_t *d_counts, int32_t vocab, int64_t inc, const int32_t *d_syms, int64_t sym_stride,
+                           int64_t n_streams, int64_t T, const int32_t *d_ntok, lac_enc_state *d_state,
+                           uint8_t *d_out, int64_t out_stride, int finish, int prec, void *stream);
+int lac_ac_decode_adaptive(int64_t *d_counts, int32_t vocab, int64_t inc, int64_t n_streams, int64_t T,
+                           const int32_t *d_ntok, lac_dec_state *d_state, const uint8_t *d_bytes,
+                           const int64_t *d_offsets, int32_t *d_syms, int64_t sym_stride, int prec, void *stream);
+int lac_acs_encode_adaptive(int64_t *d_counts, int32_t vocab, int64_t inc, const int32_t *d_syms, int64_t sym_stride,
+                            int64_t n_streams, int64_t T, const int32_t *d_ntok, lac_enc_state *d_state,
+                            uint8_t *d_out, int64_t out_stride, int finish, int prec, void *stream);
+int lac_acs_decode_adaptive(int64_t *d_counts, int32_t vocab, int64_t inc, int64_t n_streams, int64_t T,
+                            const int32_t *d_ntok, lac_dec_state *d_state, const uint8_t *d_bytes,
+                            const int64_t *d_offsets, int32_t *d_syms, int64_t sym_stride, int prec, void *stream);
 
 /* ------------------------------------------------------------------------------------
  * Host-buffer convenience calls (what bench.py's `e2e` times): pinned or pageable HOST

@@ -15,7 +15,8 @@ LIB_PATH = os.path.join(_HERE, "_lib", "liblac_b200.so")
 LAC_OK, LAC_E_ARG, LAC_E_CUDA, LAC_E_CAP, LAC_E_SYMBOL, LAC_E_STREAM = 0, -1, -2, -3, -4, -5
 LAC_ST_CAP, LAC_ST_SYMBOL, LAC_ST_TABLE, LAC_ST_TRUNC = 1, 2, 4, 8
 LAC_F_WRAP64 = 1
-ABI_VERSION = 2
+LAC_ADAPTIVE_MAX_VOCAB = 4096
+ABI_VERSION = 3
 
 
 class LacError(RuntimeError):
@@ -60,6 +61,10 @@ SIGNATURES = {
     "lac_ac_decode_tables": [_p, _i32, _i64, _i64, _p, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i64, _int, _int, _p],
     "lac_acs_encode_tables": [_p, _i32, _i64, _i64, _p, _i64, _i64, _i64, _p, _p, _p, _i64, _int, _int, _p],
     "lac_acs_decode_tables": [_p, _i32, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i64, _int, _p],
+    "lac_ac_encode_adaptive": [_p, _i32, _i64, _p, _i64, _i64, _i64, _p, _p, _p, _i64, _int, _int, _p],
+    "lac_ac_decode_adaptive": [_p, _i32, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i64, _int, _p],
+    "lac_acs_encode_adaptive": [_p, _i32, _i64, _p, _i64, _i64, _i64, _p, _p, _p, _i64, _int, _int, _p],
+    "lac_acs_decode_adaptive": [_p, _i32, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i64, _int, _p],
     "lac_encode_logits_host": [_p, _p, _i64, _i64, _i32, _p, _i64, _p, _int],
     "lac_decode_logits_host": [_p, _i64, _i64, _i32, _p, _p, _p, _int],
 }

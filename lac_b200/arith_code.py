@@ -3,6 +3,8 @@ meaning), with the coding done by the CUDA library through the C ABI.
 
 What maps to what (pramasoul/lac arith_code.py):
     Predictor / CDFPredictor / ProbPredictor   :64-135   table providers: .dist, .minp, .accept(), .copy()
+    CountPredictor                             (new)     ProbPredictor with prob(s) = counts[s], coded adaptively on
+                                                         the device
     AC(predictor, prec).to_bin / .from_bin     :144-155
     A_to_bin                                   :156-246  incremental (__call__, step, flush, info, certain, ...) and
                                                          whole-sequence (run, encode, bits, compress) coding
@@ -119,6 +121,47 @@ class ProbPredictor(CDFPredictor):
         return self
 
 
+class CountPredictor(ProbPredictor):
+    """The adaptive frequency model: prob(s) = counts[s] (ones by default), and accept(s) adds `inc` to counts[s].
+    CountPredictor(256) is the byte model of the goldens ac_adaptive.npz and acs_64k.npz.  A_to_bin.compress /
+    encode / bits and A_from_bin.decompress code a whole sequence in one adaptive kernel call (lac_ac_encode_adaptive
+    / lac_ac_decode_adaptive, counts on the device) when the counts fit the device bounds: n <= 4096, counts >= 0,
+    inc >= 0 and a total that stays below 2^62; otherwise they take the table path.  Afterwards `counts` are those
+    the predictor holds after accepting every coded symbol."""
+
+    def __init__(self, n: int, counts=None, inc: int = 1):
+        super().__init__(n)
+        self.counts = [1] * n if counts is None else [int(c) for c in counts]
+        if len(self.counts) != n:
+            raise ValueError(f"{len(self.counts)} counts for {n} symbols")
+        self.inc = int(inc)
+
+    def prob(self, symbol):
+        return self.counts[symbol]
+
+    def accept(self, symbol):
+        self.counts[symbol] += self.inc
+        self.dcache = None
+
+
+def _counts_fit(predictor, T: int, wrap64: bool) -> bool:
+    """Whether T symbols of a CountPredictor stay inside the adaptive kernels' bounds (else: the table path)."""
+    from ._ffi import LAC_ADAPTIVE_MAX_VOCAB
+    c = predictor.counts
+    return (not wrap64 and 1 <= predictor.n <= LAC_ADAPTIVE_MAX_VOCAB and predictor.inc >= 0 and min(c) >= 0
+            and sum(c) + predictor.inc * T < 1 << 62)
+
+
+def _device_counts(predictor):
+    from . import coder
+    return coder.Counts(1, predictor.n, init=np.asarray(predictor.counts, dtype=np.int64), inc=predictor.inc)
+
+
+def _take_counts(predictor, counts):
+    predictor.counts = [int(c) for c in counts.counts[0].cpu().tolist()]
+    predictor.dcache = None
+
+
 def materialise_tables(predictor, symbols: Sequence[int]):
     """Walk a predictor along `symbols` exactly as A_to_bin.receive_symbol does (table, then accept):
     returns (dist int64 [T, V], minp int64 [T])."""
@@ -161,6 +204,8 @@ def _bits_of(data: bytes, nbits: int) -> List[int]:
 def _kind(predictor) -> str:
     if type(predictor) is Predictor:
         return "uniform"
+    if type(predictor) is CountPredictor:  # whole sequences: one adaptive call; one symbol at a time: its table
+        return "counts"
     if hasattr(predictor, "logits_row"):     # llama_compress.Llama_AC: fp32 logits -> LQ32 on the device
         return "logits"
     return "tables"
@@ -405,6 +450,10 @@ class A_to_bin:
                 self.predictor.accept(s)
             enc.encode_logits(torch.stack(rows).unsqueeze(0), torch.tensor([symbols], dtype=torch.int32, device="cuda"),
                               finish=bool(stop))
+        elif kind == "counts" and _counts_fit(self.predictor, T, self.wrap64):
+            counts = _device_counts(self.predictor)
+            enc.encode_adaptive(torch.tensor([symbols], dtype=torch.int32, device="cuda"), counts, finish=bool(stop))
+            _take_counts(self.predictor, counts)
         else:
             dist, minp = materialise_tables(self.predictor, symbols)
             enc.encode_tables(torch.from_numpy(dist).cuda(), torch.tensor([symbols], dtype=torch.int32, device="cuda"),
@@ -526,6 +575,11 @@ class A_from_bin:
         kind = _kind(self.predictor)
         if kind == "uniform":
             return dec.decode_uniform(self.predictor.n, count).cpu().numpy()[0].astype(int).tolist()
+        if kind == "counts" and _counts_fit(self.predictor, count, self.wrap64):
+            counts = _device_counts(self.predictor)
+            syms = dec.decode_adaptive(counts, count).cpu().numpy()[0].astype(int).tolist()
+            _take_counts(self.predictor, counts)
+            return syms
         out: List[int] = []
         static = kind == "tables" and (not hasattr(self.predictor, "dcache")
                                        or type(self.predictor).accept is Predictor.accept)

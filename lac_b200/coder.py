@@ -96,6 +96,44 @@ def cdf_to_dist(cum: torch.Tensor) -> np.ndarray:
 
 
 # ------------------------------------------------------------------------------------ (b) coder
+class Counts:
+    """Device-resident counts of an adaptive frequency model, int64 [n_streams, vocab]: prob(s) = counts[s], and
+    every coded or decoded token adds `inc` to its symbol's count (the kernels update them in place).  `init` is
+    None (all ones), [vocab] (the same for every stream) or [n_streams, vocab].  An encoder and a decoder each need
+    their own Counts, started from the same values."""
+
+    def __init__(self, n_streams: int, vocab: int, init=None, inc: int = 1, device="cuda"):
+        self.n, self.vocab, self.inc = int(n_streams), int(vocab), int(inc)
+        if not 1 <= self.vocab <= _ffi.LAC_ADAPTIVE_MAX_VOCAB:
+            raise LacError(_ffi.LAC_E_ARG, f"vocab {self.vocab} out of range [1, {_ffi.LAC_ADAPTIVE_MAX_VOCAB}]")
+        if self.inc < 0:
+            raise LacError(_ffi.LAC_E_ARG, f"inc must be >= 0, got {self.inc}")
+        self.device = torch.device(device)
+        self.counts = torch.empty((self.n, self.vocab), dtype=torch.int64, device=self.device)
+        self.reset(init)
+
+    def reset(self, init=None):
+        """Start again from `init` (None: all ones) in the same device buffer."""
+        if init is None:
+            self.counts.fill_(1)
+            return
+        a = torch.as_tensor(np.asarray(init, dtype=np.int64) if not torch.is_tensor(init) else init)
+        if tuple(a.shape) not in ((self.vocab,), (self.n, self.vocab)):
+            raise LacError(_ffi.LAC_E_ARG, f"init must be [{self.vocab}] or [{self.n}, {self.vocab}], "
+                                           f"got {list(a.shape)}")
+        self.counts.copy_(a.to(device=self.device, dtype=torch.int64).expand(self.n, self.vocab))
+
+    @property
+    def ptr(self):
+        return self.counts.data_ptr()
+
+
+def _check_counts(counts: "Counts", n: int):
+    _need_cuda(counts.counts, "counts", torch.int64)
+    if tuple(counts.counts.shape) != (n, counts.vocab):
+        raise LacError(_ffi.LAC_E_ARG, f"counts hold {counts.counts.shape[0]} streams, the coder {n}")
+
+
 def _collect_streams(out: torch.Tensor, state: torch.Tensor) -> Tuple[List[bytes], np.ndarray]:
     st = state.cpu().numpy().view(np.uint8).reshape(-1, _ffi.ENC_STATE_BYTES)
     nbits = st[:, 16:24].copy().view(np.uint64).reshape(-1)
@@ -205,6 +243,34 @@ class StreamEncoder:
         check(lib().lac_acs_encode_tables(cdf.data_ptr(), V, ss, ts, syms.data_ptr(), T, S, T, self._ntok(ntok),
                                           self.state.data_ptr(), self.out.data_ptr(), self.cap,
                                           2 if finish == "safe" else int(bool(finish)), self.prec, _cur_stream()))
+        self.finished = self.finished or bool(finish)
+
+    def encode_adaptive(self, syms: torch.Tensor, counts: Counts, ntok: Optional[torch.Tensor] = None,
+                        finish: bool = False):
+        """Adaptive frequency model under A_to_bin: CDFPredictor on dist = cumsum(counts) before each token, then
+        counts[sym] += counts.inc (lac_ac_encode_adaptive).  syms [n_streams, T] int32; `counts` carries over
+        between calls like the coder state."""
+        _need_cuda(syms, "syms", torch.int32)
+        S, T = syms.shape
+        _check_counts(counts, self.n)
+        if S != self.n:
+            raise LacError(_ffi.LAC_E_ARG, "syms must be [n_streams, T]")
+        check(lib().lac_ac_encode_adaptive(counts.ptr, counts.vocab, counts.inc, syms.data_ptr(), T, S, T,
+                                           self._ntok(ntok), self.state.data_ptr(), self.out.data_ptr(), self.cap,
+                                           int(finish), self.prec, _cur_stream()))
+        self.finished = self.finished or finish
+
+    def acs_encode_adaptive(self, syms: torch.Tensor, counts: Counts, ntok: Optional[torch.Tensor] = None,
+                            finish=False):
+        """The same model under ACSampler (cdf = cumsum(counts)); finish as acs_encode_tables."""
+        _need_cuda(syms, "syms", torch.int32)
+        S, T = syms.shape
+        _check_counts(counts, self.n)
+        if S != self.n:
+            raise LacError(_ffi.LAC_E_ARG, "syms must be [n_streams, T]")
+        check(lib().lac_acs_encode_adaptive(counts.ptr, counts.vocab, counts.inc, syms.data_ptr(), T, S, T,
+                                            self._ntok(ntok), self.state.data_ptr(), self.out.data_ptr(), self.cap,
+                                            2 if finish == "safe" else int(bool(finish)), self.prec, _cur_stream()))
         self.finished = self.finished or bool(finish)
 
     def acs_flush(self, safe: bool = False):
@@ -362,6 +428,33 @@ class StreamDecoder:
                                           ntok.data_ptr() if ntok is not None else None, self.state.data_ptr(),
                                           self.bytes.data_ptr(), self.offsets.data_ptr(), syms.data_ptr(), T,
                                           self.prec, _cur_stream()))
+        if check_status:
+            self._check_status()
+        return syms
+
+    def decode_adaptive(self, counts: Counts, T: int, ntok: Optional[torch.Tensor] = None,
+                        check_status: bool = True) -> torch.Tensor:
+        """Decoder for encode_adaptive streams: T symbols per stream from the bits alone, `counts` (the decoder's
+        own, started where the encoder's started) updated after every symbol."""
+        _check_counts(counts, self.n)
+        syms = torch.zeros((self.n, T), dtype=torch.int32, device=self.device)
+        check(lib().lac_ac_decode_adaptive(counts.ptr, counts.vocab, counts.inc, self.n, T,
+                                           ntok.data_ptr() if ntok is not None else None, self.state.data_ptr(),
+                                           self.bytes.data_ptr(), self.offsets.data_ptr(), syms.data_ptr(), T,
+                                           self.prec, _cur_stream()))
+        if check_status:
+            self._check_status()
+        return syms
+
+    def acs_decode_adaptive(self, counts: Counts, T: int, ntok: Optional[torch.Tensor] = None,
+                            check_status: bool = True) -> torch.Tensor:
+        """Decoder for acs_encode_adaptive streams."""
+        _check_counts(counts, self.n)
+        syms = torch.zeros((self.n, T), dtype=torch.int32, device=self.device)
+        check(lib().lac_acs_decode_adaptive(counts.ptr, counts.vocab, counts.inc, self.n, T,
+                                            ntok.data_ptr() if ntok is not None else None, self.state.data_ptr(),
+                                            self.bytes.data_ptr(), self.offsets.data_ptr(), syms.data_ptr(), T,
+                                            self.prec, _cur_stream()))
         if check_status:
             self._check_status()
         return syms

@@ -248,6 +248,66 @@ int lac_acs_decode_tables(const uint64_t* d_cdf, int32_t vocab, int64_t stream_s
     return LAC_OK;
 }
 
+namespace {
+// what the four adaptive entry points check before any CUDA call
+int check_adaptive(const char* fn, const int64_t* d_counts, int32_t vocab, int64_t inc, int prec) {
+    if (!d_counts || vocab < 1 || vocab > LAC_ADAPTIVE_MAX_VOCAB || inc < 0) return fail(LAC_E_ARG, "%s: bad argument", fn);
+    if (!prec_ok(prec, 2)) return fail(LAC_E_ARG, "%s: prec %d outside [2, 60]", fn, prec);
+    return LAC_OK;
+}
+}  // namespace
+
+int lac_ac_encode_adaptive(int64_t* d_counts, int32_t vocab, int64_t inc, const int32_t* d_syms, int64_t sym_stride,
+                           int64_t n_streams, int64_t T, const int32_t* d_ntok, lac_enc_state* d_state,
+                           uint8_t* d_out, int64_t out_stride, int finish, int prec, void* stream) {
+    if ((!d_syms && T > 0) || !d_state || !d_out || n_streams < 0 || T < 0 || out_stride < 1)
+        return fail(LAC_E_ARG, "lac_ac_encode_adaptive: bad argument");
+    if (int rc = check_adaptive("lac_ac_encode_adaptive", d_counts, vocab, inc, prec)) return rc;
+    CK(lac::launch_table_encode(lac::Adaptive{vocab, d_counts, inc}, d_syms, sym_stride, n_streams, T, d_ntok, d_state,
+                                d_out, out_stride, finish ? lac::kFlushAc : lac::kFlushNone, prec,
+                                (cudaStream_t)stream),
+       "lac_ac_encode_adaptive");
+    return LAC_OK;
+}
+
+int lac_ac_decode_adaptive(int64_t* d_counts, int32_t vocab, int64_t inc, int64_t n_streams, int64_t T,
+                           const int32_t* d_ntok, lac_dec_state* d_state, const uint8_t* d_bytes,
+                           const int64_t* d_offsets, int32_t* d_syms, int64_t sym_stride, int prec, void* stream) {
+    if (!d_state || !d_bytes || !d_offsets || !d_syms || n_streams < 0 || T < 0)
+        return fail(LAC_E_ARG, "lac_ac_decode_adaptive: bad argument");
+    if (int rc = check_adaptive("lac_ac_decode_adaptive", d_counts, vocab, inc, prec)) return rc;
+    CK(lac::launch_table_decode(lac::Adaptive{vocab, d_counts, inc}, n_streams, T, d_ntok, d_state, d_bytes, d_offsets,
+                                d_syms, sym_stride, prec, (cudaStream_t)stream),
+       "lac_ac_decode_adaptive");
+    return LAC_OK;
+}
+
+int lac_acs_encode_adaptive(int64_t* d_counts, int32_t vocab, int64_t inc, const int32_t* d_syms, int64_t sym_stride,
+                            int64_t n_streams, int64_t T, const int32_t* d_ntok, lac_enc_state* d_state,
+                            uint8_t* d_out, int64_t out_stride, int finish, int prec, void* stream) {
+    if ((!d_syms && T > 0) || !d_state || !d_out || n_streams < 0 || T < 0 || out_stride < 1)
+        return fail(LAC_E_ARG, "lac_acs_encode_adaptive: bad argument");
+    if (int rc = check_adaptive("lac_acs_encode_adaptive", d_counts, vocab, inc, prec)) return rc;
+    // finish 1: flush_compress (the reference's), 2: the safe termination, anything else: no flush
+    const int flush = finish == 1 ? lac::kFlushCompress : (finish == 2 ? lac::kFlushAc : lac::kFlushNone);
+    CK(lac::launch_table_encode(lac::AcsAdaptive{vocab, d_counts, inc}, d_syms, sym_stride, n_streams, T, d_ntok,
+                                d_state, d_out, out_stride, flush, prec, (cudaStream_t)stream),
+       "lac_acs_encode_adaptive");
+    return LAC_OK;
+}
+
+int lac_acs_decode_adaptive(int64_t* d_counts, int32_t vocab, int64_t inc, int64_t n_streams, int64_t T,
+                            const int32_t* d_ntok, lac_dec_state* d_state, const uint8_t* d_bytes,
+                            const int64_t* d_offsets, int32_t* d_syms, int64_t sym_stride, int prec, void* stream) {
+    if (!d_state || !d_bytes || !d_offsets || !d_syms || n_streams < 0 || T < 0)
+        return fail(LAC_E_ARG, "lac_acs_decode_adaptive: bad argument");
+    if (int rc = check_adaptive("lac_acs_decode_adaptive", d_counts, vocab, inc, prec)) return rc;
+    CK(lac::launch_table_decode(lac::AcsAdaptive{vocab, d_counts, inc}, n_streams, T, d_ntok, d_state, d_bytes,
+                                d_offsets, d_syms, sym_stride, prec, (cudaStream_t)stream),
+       "lac_acs_decode_adaptive");
+    return LAC_OK;
+}
+
 // ------------------------------------------------------------------ host-buffer calls
 namespace {
 

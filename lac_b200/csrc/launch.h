@@ -78,6 +78,20 @@ struct Acs {  // ACSampler: table (s, t) at cdf + s * ss + t * ts
     const uint64_t* cdf;
     int64_t ss, ts;
 };
+// Adaptive count models, prob(s) = counts[s] and counts[sym] += inc after every token; the counts of stream s at
+// counts + s * n_symbols (n_symbols <= LAC_ADAPTIVE_MAX_VOCAB), read at the start of a call and written back at its end
+struct Adaptive {  // CDFPredictor semantics (ProbPredictor under A_to_bin / A_from_bin)
+    static constexpr int kEncLanes = 32, kDecLanes = 32;
+    int n_symbols;
+    int64_t* counts;
+    int64_t inc;
+};
+struct AcsAdaptive {  // ACSampler semantics
+    static constexpr int kEncLanes = 32, kDecLanes = 32;
+    int n_symbols;
+    int64_t* counts;
+    int64_t inc;
+};
 // how an encode call ends a stream: A_to_bin.flush (coder::ac_flush) or ACSampler's flush_compress
 enum TableFlush { kFlushNone, kFlushAc, kFlushCompress };
 template <class Model>

@@ -13,6 +13,9 @@
 //            which holds for arbitrary f_i (also the wrapped int64 products of Llama_AC, flag LAC_F_WRAP64).
 //   Acs      ACSampler / Region semantics (arithmetic_coding.py) on uint64 tables: one thread per stream encodes,
 //            one warp per stream decodes.
+//   Adaptive, AcsAdaptive   adaptive count models, prob(s) = counts[s] with counts[sym] += inc after every token, on
+//            the Cdf resp. Acs arithmetic; one warp per stream keeps the stream's table in shared memory (the
+//            per-stream hooks stream_begin / stream_accept / stream_end, empty for the static models).
 // The models' data are in launch.h; range(m, ...) and symbol(m, ...) below are their device side.  Both return false,
 // coding nothing, for a token the model cannot code (LAC_ST_TABLE).
 #include <cstdint>
@@ -199,11 +202,9 @@ __device__ __forceinline__ bool symbol(const Cdf& m, int64_t s, int64_t t, int64
 // ------------------------------------------------------------------ ACSampler on tables
 // The token of the sample_scaled_cdf compress path (arithmetic_coding.py:85-87) narrows the region as Region.step does
 // (arithmetic_coding.py:160-168): map(v, d) = low + span * v // d, the new region [map(c[i-1]), map(c[i]) - 1].  An
-// empty region is LAC_ST_TABLE: the reference would never terminate.
-__device__ __forceinline__ bool range(const Acs& m, int64_t s, int64_t t, int tok, int64_t w, int, int64_t& r0,
-                                      int64_t& r1) {
-    const uint64_t* c = m.cdf + s * m.ss + t * m.ts;
-    const uint64_t cl = tok ? c[tok - 1] : 0, ch = c[tok], den = c[m.n_symbols - 1];
+// empty region is LAC_ST_TABLE: the reference would never terminate.  c is one inclusive table of V entries.
+__device__ __forceinline__ bool acs_range(const uint64_t* c, int V, int tok, int64_t w, int64_t& r0, int64_t& r1) {
+    const uint64_t cl = tok ? c[tok - 1] : 0, ch = c[tok], den = c[V - 1];
     if (den == 0 || ch <= cl) return false;
     const u128 span = (u128)(uint64_t)w;
     r0 = (int64_t)(uint64_t)((span * cl) / den);
@@ -212,21 +213,169 @@ __device__ __forceinline__ bool range(const Acs& m, int64_t s, int64_t t, int to
 }
 // The symbol whose encoder interval [map(c[i-1]), map(c[i]) - 1] contains the value:
 // map(c) <= v  <=>  c <= ceil((v - low + 1) * den / span) - 1.  No zero-width check: that symbol holds the value.
-__device__ __forceinline__ bool symbol(const Acs& m, int64_t s, int64_t t, int64_t x, int64_t w, int lane, int& tok,
-                                       int64_t& r0, int64_t& r1) {
-    const uint64_t* c = m.cdf + s * m.ss + t * m.ts;
-    const uint64_t den = c[m.n_symbols - 1];
+__device__ __forceinline__ bool acs_symbol(const uint64_t* c, int V, int64_t x, int64_t w, int lane, int& tok,
+                                           int64_t& r0, int64_t& r1) {
+    const uint64_t den = c[V - 1];
     if (den == 0) return false;
     const u128 span = (u128)(uint64_t)w;
     const u128 tau = ((u128)(uint64_t)(x + 1) * den + span - 1) / span - 1;
     int64_t cnt = 0;
-    for (int i = lane; i < m.n_symbols; i += 32) cnt += ((u128)c[i] <= tau);
+    for (int i = lane; i < V; i += 32) cnt += ((u128)c[i] <= tau);
     tok = (int)warp_sum_i64(cnt);
-    if (tok >= m.n_symbols) return false;
+    if (tok >= V) return false;
     const uint64_t cl = tok ? c[tok - 1] : 0, ch = c[tok];
     r0 = (int64_t)(uint64_t)((span * cl) / den);
     r1 = (int64_t)(uint64_t)((span * ch) / den);
     return true;
+}
+
+__device__ __forceinline__ bool range(const Acs& m, int64_t s, int64_t t, int tok, int64_t w, int, int64_t& r0,
+                                      int64_t& r1) {
+    return acs_range(m.cdf + s * m.ss + t * m.ts, m.n_symbols, tok, w, r0, r1);
+}
+__device__ __forceinline__ bool symbol(const Acs& m, int64_t s, int64_t t, int64_t x, int64_t w, int lane, int& tok,
+                                       int64_t& r0, int64_t& r1) {
+    return acs_symbol(m.cdf + s * m.ss + t * m.ts, m.n_symbols, x, w, lane, tok, r0, r1);
+}
+
+// ------------------------------------------------------------------ adaptive count models
+// prob(s) = counts[s], and after every token counts[sym] += inc (a ProbPredictor whose accept() counts).  The warp of
+// a stream keeps the stream's table in shared memory as int64 inclusive cumulative values -- exactly the table the
+// reference predictor builds before each token -- so the range and symbol arithmetic is that of the static models on
+// the shared table: Adaptive is CDFPredictor (fudged_dist included, minp = the smallest positive count), AcsAdaptive
+// is ACSampler.  Totals stay below 2^62 (kAdaptiveTotal): a token whose accept() would reach it is LAC_ST_TABLE.
+constexpr int64_t kAdaptiveTotal = 1ll << 62;
+
+__device__ __forceinline__ int64_t warp_min_i64(int64_t v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        int64_t t = __shfl_xor_sync(0xffffffffu, v, o);
+        v = t < v ? t : v;
+    }
+    return v;
+}
+
+// One stream of an adaptive model M, as the drivers see it between begin and end.
+template <class M>
+struct CountTable {
+    int64_t* tbl;     // shared: the stream's inclusive cumulative counts
+    int64_t* counts;  // global: the stream's counts, read at begin, written at end
+    int V;
+    int64_t inc;
+    bool loaded;      // false: a count was negative or the total reached kAdaptiveTotal; nothing is coded or stored
+};
+
+// Load the stream's counts into its shared table, 32 at a time: a warp scan of each chunk plus the running total.
+// Sums saturate at kAdaptiveTotal, so a table that reaches it (and is rejected) cannot overflow on the way.
+template <class M>
+__device__ inline CountTable<M> count_table(const M& m, int64_t s, int lane) {
+    extern __shared__ int64_t count_tables[];  // one table of V entries per warp of the block (count_shape)
+    CountTable<M> a;
+    a.V = m.n_symbols;
+    a.inc = m.inc;
+    a.tbl = count_tables + (int64_t)(threadIdx.x / 32) * a.V;
+    a.counts = m.counts + s * a.V;
+    const uint64_t lim = (uint64_t)kAdaptiveTotal;
+    uint64_t run = 0;
+    bool bad = false;
+    for (int b = 0; b < a.V; b += 32) {
+        const int i = b + lane;
+        const int64_t c = i < a.V ? a.counts[i] : 0;
+        bad |= c < 0;
+        uint64_t v = c < 0 ? 0 : ((uint64_t)c < lim ? (uint64_t)c : lim);
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint64_t u = __shfl_up_sync(0xffffffffu, v, o);
+            if (lane >= o) v = v + u < lim ? v + u : lim;
+        }
+        v = v + run < lim ? v + run : lim;
+        if (i < a.V) a.tbl[i] = (int64_t)v;
+        run = __shfl_sync(0xffffffffu, v, 31);
+    }
+    a.loaded = !__any_sync(0xffffffffu, bad) && run < lim;
+    __syncwarp();
+    return a;
+}
+
+// CDFPredictor on the shared table.  minp only matters once the total exceeds the width (fudged_dist needs
+// total > w * minp, and minp >= 1), so the warp looks for the smallest positive count only then.
+template <class M>
+__device__ __forceinline__ TableCtx count_ctx(const CountTable<M>& a, int64_t w, int lane) {
+    TableCtx c;
+    c.tbl = a.tbl;
+    c.V = a.V;
+    c.minp = 1;
+    c.wrap = 0;
+    if (a.tbl[a.V - 1] > w) {
+        int64_t mn = kAdaptiveTotal;
+        for (int i = lane; i < a.V; i += 32) {
+            const int64_t f = a.tbl[i] - (i ? a.tbl[i - 1] : 0);
+            if (f > 0 && f < mn) mn = f;
+        }
+        c.minp = warp_min_i64(mn);
+    }
+    return c;
+}
+// room for this token's accept() below kAdaptiveTotal
+template <class M>
+__device__ __forceinline__ bool count_room(const CountTable<M>& a) {
+    return a.tbl[a.V - 1] < kAdaptiveTotal - a.inc;
+}
+
+__device__ __forceinline__ bool range(const CountTable<Adaptive>& a, int64_t, int64_t, int sym, int64_t w, int lane,
+                                      int64_t& r0, int64_t& r1) {
+    return count_room(a) && table_range(count_ctx(a, w, lane), sym, w, lane, r0, r1);
+}
+__device__ __forceinline__ bool symbol(const CountTable<Adaptive>& a, int64_t, int64_t, int64_t x, int64_t w, int lane,
+                                       int& sym, int64_t& r0, int64_t& r1) {
+    if (!count_room(a)) return false;
+    const TableCtx c = count_ctx(a, w, lane);
+    sym = table_symbol(c, x, w, lane);
+    return sym < a.V && table_range(c, sym, w, lane, r0, r1);
+}
+__device__ __forceinline__ bool range(const CountTable<AcsAdaptive>& a, int64_t, int64_t, int tok, int64_t w, int,
+                                      int64_t& r0, int64_t& r1) {
+    return count_room(a) && acs_range((const uint64_t*)a.tbl, a.V, tok, w, r0, r1);
+}
+__device__ __forceinline__ bool symbol(const CountTable<AcsAdaptive>& a, int64_t, int64_t, int64_t x, int64_t w,
+                                       int lane, int& tok, int64_t& r0, int64_t& r1) {
+    return count_room(a) && acs_symbol((const uint64_t*)a.tbl, a.V, x, w, lane, tok, r0, r1);
+}
+
+// ------------------------------------------------------------------ per-stream model hooks
+// stream_begin(m, s, lane) gives what range / symbol work on for stream s: the model itself for the static models,
+// whose other hooks are empty, and the stream's shared table for the adaptive ones.  stream_accept follows every token
+// that narrowed the interval, stream_end the last one.  Every lane of a stream calls every hook.
+template <class M>
+__device__ __forceinline__ const M& stream_begin(const M& m, int64_t, int) { return m; }
+template <class M>
+__device__ __forceinline__ bool stream_loaded(const M&) { return true; }
+template <class M>
+__device__ __forceinline__ void stream_accept(const M&, int, int) {}
+template <class M>
+__device__ __forceinline__ void stream_end(const M&, int) {}
+
+__device__ __forceinline__ CountTable<Adaptive> stream_begin(const Adaptive& m, int64_t s, int lane) {
+    return count_table(m, s, lane);
+}
+__device__ __forceinline__ CountTable<AcsAdaptive> stream_begin(const AcsAdaptive& m, int64_t s, int lane) {
+    return count_table(m, s, lane);
+}
+template <class M>
+__device__ __forceinline__ bool stream_loaded(const CountTable<M>& a) { return a.loaded; }
+// counts[sym] += inc: entries sym .. V-1 of the cumulative table
+template <class M>
+__device__ __forceinline__ void stream_accept(const CountTable<M>& a, int sym, int lane) {
+    if (a.inc == 0) return;
+    __syncwarp();  // every lane has read this token's table
+    for (int i = sym + lane; i < a.V; i += 32) a.tbl[i] += a.inc;
+    __syncwarp();
+}
+// the table goes back as counts
+template <class M>
+__device__ __forceinline__ void stream_end(const CountTable<M>& a, int lane) {
+    if (!a.loaded) return;
+    for (int i = lane; i < a.V; i += 32) a.counts[i] = a.tbl[i] - (i ? a.tbl[i - 1] : 0);
 }
 
 // ------------------------------------------------------------------ drivers
@@ -243,7 +392,8 @@ __global__ void table_encode_kernel(const Model m, const int32_t* __restrict__ s
     int64_t l = state[s].low, h = state[s].high;
     coder::BitWriter bw;
     bw.open(out + s * out_stride, (uint64_t)out_stride, state[s].nbits, state[s].status);
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
+    const auto& ms = stream_begin(m, s, lane);  // a stream whose table does not load codes nothing: LAC_ST_TABLE
+    const int64_t Ts = !stream_loaded(ms) ? 0 : ntok ? (int64_t)ntok[s] : T;
     for (int64_t t = 0; t < Ts; t++) {
         const int sym = syms[s * sym_stride + t];
         if (sym < 0 || sym >= m.n_symbols) {
@@ -251,12 +401,13 @@ __global__ void table_encode_kernel(const Model m, const int32_t* __restrict__ s
             break;
         }
         int64_t r0, r1;
-        if (!range(m, s, t, sym, h - l + 1, lane, r0, r1)) {
+        if (!range(ms, s, t, sym, h - l + 1, lane, r0, r1)) {
             bw.status |= LAC_ST_TABLE;
             break;
         }
         h = l + r1 - 1;  // receive_symbol :169-175
         l += r0;
+        stream_accept(ms, sym, lane);
         const int k = coder::renorm_count((uint64_t)(h - l + 1), P);
         const int64_t E = coder::renorm_apply(l, h, P, k);
         if (lane == 0) bw.append(E, k);
@@ -264,6 +415,8 @@ __global__ void table_encode_kernel(const Model m, const int32_t* __restrict__ s
         if constexpr (LANES > 1) st = __shfl_sync(0xffffffffu, st, 0);
         if (st & LAC_ST_CAP) break;
     }
+    if (!stream_loaded(ms)) bw.status |= LAC_ST_TABLE;
+    stream_end(ms, lane);
     if (lane != 0) return;
     if (flush != kFlushNone && !(bw.status & (LAC_ST_TABLE | LAC_ST_SYMBOL | LAC_ST_CAP))) {
         if (flush == kFlushCompress) {
@@ -305,16 +458,18 @@ __global__ void table_decode_kernel(const Model m, int64_t n_streams, int64_t T,
     uint32_t status = state[s].status;
     const uint8_t* data = bytes + offsets[s];
     const uint64_t nbytes = (uint64_t)(offsets[s + 1] - offsets[s]);
-    const int64_t Ts = ntok ? (int64_t)ntok[s] : T;
+    const auto& ms = stream_begin(m, s, lane);  // a stream whose table does not load decodes nothing: LAC_ST_TABLE
+    const int64_t Ts = !stream_loaded(ms) ? 0 : ntok ? (int64_t)ntok[s] : T;
     for (int64_t t = 0; t < Ts; t++) {
         int sym;
         int64_t r0, r1;
-        if (!symbol(m, s, t, v - l, h - l + 1, lane, sym, r0, r1)) {
+        if (!symbol(ms, s, t, v - l, h - l + 1, lane, sym, r0, r1)) {
             status |= LAC_ST_TABLE;
             break;
         }
         h = l + r1 - 1;
         l += r0;
+        stream_accept(ms, sym, lane);
         const int64_t off = v - l;
         const int k = coder::renorm_count((uint64_t)(h - l + 1), P);
         coder::renorm_apply(l, h, P, k);
@@ -322,6 +477,8 @@ __global__ void table_decode_kernel(const Model m, int64_t n_streams, int64_t T,
         pos += (uint64_t)k;
         if (lane == 0) syms[s * sym_stride + t] = sym;
     }
+    if (!stream_loaded(ms)) status |= LAC_ST_TABLE;
+    stream_end(ms, lane);
     if (lane == 0) {
         state[s].low = l;
         state[s].high = h;
@@ -332,15 +489,41 @@ __global__ void table_decode_kernel(const Model m, int64_t n_streams, int64_t T,
 }
 
 // ------------------------------------------------------------------ launchers
-// One lane per stream: blocks of 32 threads.  32 lanes per stream: blocks of 128 threads, 4 streams per block.
+// One lane per stream: blocks of 32 threads.  32 lanes per stream: blocks of 128 threads, 4 streams per block.  The
+// adaptive models keep a V-entry int64 table per stream in dynamic shared memory: up to 4 streams per block within
+// 48 KB, so V = 4096 (32 KB) runs one stream per block and no block needs the opt-in above 48 KB.
+struct Shape {
+    unsigned threads;
+    size_t smem;
+};
+template <int LANES, class M>
+Shape launch_shape(const M&) {
+    return {LANES == 1 ? 32u : 128u, 0};
+}
+inline Shape count_shape(int V) {
+    const size_t per = (size_t)V * sizeof(int64_t);
+    size_t spb = (size_t(48) << 10) / per;
+    spb = spb < 1 ? 1 : (spb > 4 ? 4 : spb);
+    return {(unsigned)(32 * spb), spb * per};
+}
+template <int LANES>
+Shape launch_shape(const Adaptive& m) {
+    return count_shape(m.n_symbols);
+}
+template <int LANES>
+Shape launch_shape(const AcsAdaptive& m) {
+    return count_shape(m.n_symbols);
+}
+
 template <class M>
 cudaError_t launch_table_encode(const M& m, const int32_t* syms, int64_t sym_stride, int64_t n, int64_t T,
                                 const int32_t* ntok, lac_enc_state* state, uint8_t* out, int64_t out_stride, int flush,
                                 int P, cudaStream_t st) {
     if (n == 0) return cudaSuccess;  // T == 0 is the flush-only call
     constexpr int lanes = M::kEncLanes;
-    constexpr unsigned threads = lanes == 1 ? 32 : 128, spb = threads / lanes;
-    table_encode_kernel<M, lanes><<<(unsigned)((n + spb - 1) / spb), threads, 0, st>>>(
+    const Shape sh = launch_shape<lanes>(m);
+    const unsigned spb = sh.threads / lanes;
+    table_encode_kernel<M, lanes><<<(unsigned)((n + spb - 1) / spb), sh.threads, sh.smem, st>>>(
         m, syms, sym_stride, n, T, ntok, state, out, out_stride, flush, P);
     return cudaGetLastError();
 }
@@ -351,8 +534,9 @@ cudaError_t launch_table_decode(const M& m, int64_t n, int64_t T, const int32_t*
                                 cudaStream_t st) {
     if (n == 0 || T == 0) return cudaSuccess;
     constexpr int lanes = M::kDecLanes;
-    constexpr unsigned threads = lanes == 1 ? 32 : 128, spb = threads / lanes;
-    table_decode_kernel<M, lanes><<<(unsigned)((n + spb - 1) / spb), threads, 0, st>>>(
+    const Shape sh = launch_shape<lanes>(m);
+    const unsigned spb = sh.threads / lanes;
+    table_decode_kernel<M, lanes><<<(unsigned)((n + spb - 1) / spb), sh.threads, sh.smem, st>>>(
         m, n, T, ntok, state, bytes, offsets, syms, sym_stride, P);
     return cudaGetLastError();
 }
@@ -365,6 +549,8 @@ cudaError_t launch_table_decode(const M& m, int64_t n, int64_t T, const int32_t*
 LAC_TABLE_CODER(Uniform)
 LAC_TABLE_CODER(Cdf)
 LAC_TABLE_CODER(Acs)
+LAC_TABLE_CODER(Adaptive)
+LAC_TABLE_CODER(AcsAdaptive)
 #undef LAC_TABLE_CODER
 
 }  // namespace lac
