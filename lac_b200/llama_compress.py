@@ -266,8 +266,8 @@ class StepEngine:
 
 
 class LlamaCompressor:
-    """compress(token ids) -> LACB bytes, decompress(bytes) -> token ids.  With torch.distributed initialised every
-    rank calls both with the same arguments; rank 0 gets the result, the others None."""
+    """compress(token ids) -> LACB bytes, decompress(bytes[, start, stop]) -> token ids.  With torch.distributed
+    initialised every rank calls both with the same arguments; rank 0 gets the result, the others None."""
 
     def __init__(self, model: LlamaModel, chunk_tokens: int = 2048, prec: int = coder.DEFAULT_PREC,
                  use_graphs: bool = True, group=None):
@@ -284,7 +284,9 @@ class LlamaCompressor:
         return sharding.compress_sharded(toks, self.chunk, self.model.S, self.engine.encode_batch, self.prec,
                                          self.vocab, self.model.device, self.tag, self.group)
 
-    def decompress(self, blob: bytes) -> Optional[np.ndarray]:
+    def decompress(self, blob: bytes, start: Optional[int] = None, stop: Optional[int] = None) -> Optional[np.ndarray]:
+        """The tokens of the file, or tokens[start:stop] (0 <= start <= stop <= total, no negative indices): only
+        the batches that hold the range are decoded, each for as many steps as its needed chunks reach into it."""
         c = container.unpack(blob)
         if c.vocab != self.vocab or c.quantiser != container.QUANT_LQ32:
             raise ValueError("container was written for a different vocabulary / quantiser")
@@ -293,7 +295,8 @@ class LlamaCompressor:
                              f"tokens; this compressor runs {self.model.S} x {self.chunk}")
         if c.tag and c.tag != self.tag:
             raise ValueError("container was written with a different predictor configuration")
-        return sharding.decompress_sharded(blob, self.engine.decode_batch, self.model.device, self.group)
+        return sharding.decompress_sharded(blob, self.engine.decode_batch, self.model.device, self.group,
+                                           0 if start is None else start, stop)
 
 
 # ------------------------------------------------------------------ the reference's own entry points

@@ -9,6 +9,7 @@ chunks, are what is dealt to the ranks: rank r owns a contiguous range of batche
 """
 from __future__ import annotations
 
+import numbers
 from typing import Callable, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -150,24 +151,58 @@ def compress_sharded(tokens, chunk_tokens: int, batch_streams: int, encode_batch
                                   quantiser, batch_streams, tag)
 
 
-def decompress_sharded(blob: bytes, decode_batch: DecodeBatch, device, group=None) -> Optional[np.ndarray]:
-    """Every rank passes the SAME file; rank 0 returns the tokens (None elsewhere)."""
+def _check_range(start, stop, total: int) -> Tuple[int, int]:
+    for name, v in (("start", start), ("stop", stop)):
+        if isinstance(v, bool) or not isinstance(v, numbers.Integral):
+            raise ValueError(f"{name} must be an integer, got {v!r}")
+    if not 0 <= start <= stop <= total:
+        raise ValueError(f"token range [{start}, {stop}) is not inside the file's [0, {total}]")
+    return int(start), int(stop)
+
+
+def decompress_sharded(blob: bytes, decode_batch: DecodeBatch, device, group=None, start: int = 0,
+                       stop: Optional[int] = None) -> Optional[np.ndarray]:
+    """Every rank passes the SAME file and range; rank 0 returns tokens[start:stop] (None elsewhere).  The default
+    range is the whole file.
+
+    Only the batches holding a chunk that overlaps [start, stop) are decoded, dealt contiguously over the ranks.  A
+    needed chunk is decoded from its first token on, min(its length, stop - its first token) tokens of its stream;
+    every other slot of the batch is an empty stream with 0 tokens.  The batch keeps its full shape, and the model
+    keeps rows independent at a fixed shape, so a needed row sees the logits it saw when the file was written
+    (tests/test_gpu_token_range.py).  A batch costs as many model steps as its longest needed prefix.  A chunk
+    with no tokens overlaps no range and is never decoded."""
     rank, world = _world(group)
     c = container.unpack(blob)
+    first = np.zeros(c.n_chunks + 1, dtype=np.int64)          # first token of every chunk, and the total
+    np.cumsum(c.ntok, out=first[1:])
+    start, stop = _check_range(start, first[-1] if stop is None else stop, int(first[-1]))
+    if start == stop:
+        return np.zeros(0, dtype=np.int32) if rank == 0 else None
+    want = np.minimum(c.ntok.astype(np.int64), np.maximum(stop - first[:-1], 0))   # tokens to decode per chunk
+    want[first[1:] <= start] = 0
+    needed = np.flatnonzero(want)
     B = c.batch_streams or max(c.n_chunks, 1)
-    spans = batch_spans(c.n_chunks, B, world)
-    b, e = spans[rank]
-    all_streams = c.streams()
-    local = np.zeros((e - b, c.chunk_tokens), dtype=np.int32)
-    for c0 in range(b, e, B):
-        c1 = min(e, c0 + B)
-        bs = all_streams[c0:c1] + [b""] * (B - (c1 - c0))
+    batches = np.unique(needed // B)
+    # rank r decodes batches[b:e], (b, e) = chunk_range(len(batches), r, world), and holds the decoded rows of
+    # needed[rows[b]:rows[e]]
+    rows = np.append(np.searchsorted(needed // B, batches), len(needed))
+    deal = [chunk_range(len(batches), r, world) for r in range(world)]
+    spans = [(int(rows[b]), int(rows[e])) for b, e in deal]
+    b, e = deal[rank]
+    off = c.offsets()
+    local = np.zeros((spans[rank][1] - spans[rank][0], c.chunk_tokens), dtype=np.int32)
+    at = 0
+    for k in batches[b:e]:
+        c0, c1 = int(k) * B, min(c.n_chunks, (int(k) + 1) * B)
+        bs = [c.payload[off[i]:off[i + 1]] if want[i] else b"" for i in range(c0, c1)] + [b""] * (B - (c1 - c0))
         bn = np.zeros(B, dtype=np.int32)
-        bn[: c1 - c0] = c.ntok[c0:c1]
-        local[c0 - b:c1 - b] = decode_batch(bs, bn)[: c1 - c0]
-    got = gather_tokens(torch.from_numpy(local).to(device), c.n_chunks, c.chunk_tokens, spans, 0, group)
+        bn[: c1 - c0] = want[c0:c1]
+        got = decode_batch(bs, bn)[: c1 - c0][want[c0:c1] > 0]
+        local[at:at + len(got)] = got
+        at += len(got)
+    got = gather_tokens(torch.from_numpy(local).to(device), len(needed), c.chunk_tokens, spans, 0, group)
     if rank != 0:
         return None
     got = got.cpu().numpy()
-    flat = [got[i, : int(c.ntok[i])] for i in range(c.n_chunks)]
-    return np.concatenate(flat) if flat else np.zeros(0, dtype=np.int32)
+    flat = np.concatenate([got[j, : want[i]] for j, i in enumerate(needed)])
+    return flat[start - first[needed[0]]:]
