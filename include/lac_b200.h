@@ -41,7 +41,7 @@
 extern "C" {
 #endif
 
-#define LAC_ABI_VERSION 3
+#define LAC_ABI_VERSION 4
 
 typedef enum {
     LAC_OK = 0,
@@ -244,6 +244,45 @@ int lac_acs_encode_adaptive(int64_t *d_counts, int32_t vocab, int64_t inc, const
 int lac_acs_decode_adaptive(int64_t *d_counts, int32_t vocab, int64_t inc, int64_t n_streams, int64_t T,
                             const int32_t *d_ntok, lac_dec_state *d_state, const uint8_t *d_bytes,
                             const int64_t *d_offsets, int32_t *d_syms, int64_t sym_stride, int prec, void *stream);
+
+/* ------------------------------------------------------------------------------------
+ * (e) batch-invariant model kernels: the layers of a Llama-style decoder (llama_compress.LlamaModel with
+ * batch_invariant=True).  bf16 activations and weights, fp32 accumulation, row-major tensors.
+ *
+ * Invariance contract: the bits of output row r depend only on row r's inputs, the weights and, for attention,
+ * the KV cache up to that row's position.  They never depend on M, on the number of query positions a launch
+ * covers, or on which CTA (or which row of a tile) computes the row.  So a prefill launch over T_blk positions
+ * of S streams (M = T_blk * S, row t * S + s) reproduces, bit for bit, the rows a per-token step computes with
+ * M = S.
+ *
+ * Activations are position-major: row r = t * S + s is stream s at position base + t, where base = *d_pos when
+ * d_pos (device, one int64) is given -- the per-token step, so one CUDA graph serves every position -- and p0
+ * otherwise.  The KV cache is [S, kv_heads, max_len, hd] bf16; qkv rows are [heads | kv_heads | kv_heads] x hd.
+ * ---------------------------------------------------------------------------------- */
+#define LAC_MODEL_OUT_BF16 0      /* y = bf16(x @ w) */
+#define LAC_MODEL_OUT_BF16_ADD 1  /* y = bf16(res + bf16(x @ w)); y may be res */
+#define LAC_MODEL_OUT_F32 2       /* y = x @ w in fp32 (the logits) */
+
+/* Y[M, N] = X[M, K] @ W[K, N] on tcgen05 (TMA ring, accumulator in tensor memory), tile 128 x 128 x 64 for every
+ * shape, K in one ascending pass.  N a multiple of 128 and K a multiple of 64 (every CONFIGS geometry); other
+ * shapes return LAC_E_ARG.  All pointers 16-byte aligned. */
+int lac_model_gemm(const void *d_x, const void *d_w, int64_t M, int32_t N, int32_t K, int epilogue,
+                   const void *d_res, void *d_y, void *stream);
+/* y = bf16(x * rsqrt(mean(x^2) + eps)) per row; dim a multiple of 256. */
+int lac_model_rmsnorm(const void *d_x, int64_t rows, int32_t dim, float eps, void *d_y, void *stream);
+/* Rotate-half RoPE of the q and k heads of every qkv row in place, from the [max_len, hd] bf16 tables, and write
+ * k and v to the cache at the row's position.  rows a multiple of n_streams. */
+int lac_model_rope_kv(void *d_qkv, int64_t rows, int32_t n_streams, int32_t heads, int32_t kv_heads, int32_t hd,
+                      const void *d_cos, const void *d_sin, const int64_t *d_pos, int64_t p0, void *d_kc,
+                      void *d_vc, int32_t max_len, void *stream);
+/* y[r, j] = bf16(bf16(silu(h[r, j])) * h[r, ffn + j]) for h [rows, 2 * ffn]. */
+int lac_model_swiglu(const void *d_h, int64_t rows, int32_t ffn, void *d_y, void *stream);
+/* Causal GQA attention of n_q query positions per stream (the roped q of qkv) over the KV cache, hd 64 or 128:
+ * out [n_q * S, heads * hd].  Each query visits 64-key blocks from slot 0 in order, fp32 online softmax with
+ * exp2, and skips per row the blocks past its position. */
+int lac_model_attention(const void *d_qkv, int32_t n_streams, int32_t n_q, int32_t heads, int32_t kv_heads,
+                        int32_t hd, const int64_t *d_pos, int64_t p0, const void *d_kc, const void *d_vc,
+                        int32_t max_len, void *d_out, void *stream);
 
 /* ------------------------------------------------------------------------------------
  * Host-buffer convenience calls (what bench.py's `e2e` times): pinned or pageable HOST

@@ -16,7 +16,8 @@ LAC_OK, LAC_E_ARG, LAC_E_CUDA, LAC_E_CAP, LAC_E_SYMBOL, LAC_E_STREAM = 0, -1, -2
 LAC_ST_CAP, LAC_ST_SYMBOL, LAC_ST_TABLE, LAC_ST_TRUNC = 1, 2, 4, 8
 LAC_F_WRAP64 = 1
 LAC_ADAPTIVE_MAX_VOCAB = 4096
-ABI_VERSION = 3
+LAC_MODEL_OUT_BF16, LAC_MODEL_OUT_BF16_ADD, LAC_MODEL_OUT_F32 = 0, 1, 2
+ABI_VERSION = 4
 
 
 class LacError(RuntimeError):
@@ -38,7 +39,7 @@ class DecState(C.Structure):
 ENC_STATE_BYTES = C.sizeof(EncState)   # 32
 DEC_STATE_BYTES = C.sizeof(DecState)   # 40
 
-_p, _i64, _i32, _int = C.c_void_p, C.c_int64, C.c_int32, C.c_int
+_p, _i64, _i32, _int, _f32 = C.c_void_p, C.c_int64, C.c_int32, C.c_int, C.c_float
 
 # name -> argtypes; every symbol include/lac_b200.h declares (tests/test_abi.py checks the set)
 SIGNATURES = {
@@ -65,6 +66,11 @@ SIGNATURES = {
     "lac_ac_decode_adaptive": [_p, _i32, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i64, _int, _p],
     "lac_acs_encode_adaptive": [_p, _i32, _i64, _p, _i64, _i64, _i64, _p, _p, _p, _i64, _int, _int, _p],
     "lac_acs_decode_adaptive": [_p, _i32, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i64, _int, _p],
+    "lac_model_gemm": [_p, _p, _i64, _i32, _i32, _int, _p, _p, _p],
+    "lac_model_rmsnorm": [_p, _i64, _i32, _f32, _p, _p],
+    "lac_model_rope_kv": [_p, _i64, _i32, _i32, _i32, _i32, _p, _p, _p, _i64, _p, _p, _i32, _p],
+    "lac_model_swiglu": [_p, _i64, _i32, _p, _p],
+    "lac_model_attention": [_p, _i32, _i32, _i32, _i32, _i32, _p, _i64, _p, _p, _i32, _p, _p],
     "lac_encode_logits_host": [_p, _p, _i64, _i64, _i32, _p, _i64, _p, _int],
     "lac_decode_logits_host": [_p, _i64, _i64, _i32, _p, _p, _p, _int],
 }

@@ -376,6 +376,64 @@ struct Pieces {
 
 }  // namespace
 
+// ---- (e) batch-invariant model kernels
+int lac_model_gemm(const void* d_x, const void* d_w, int64_t M, int32_t N, int32_t K, int epilogue,
+                   const void* d_res, void* d_y, void* stream) {
+    if (!d_x || !d_w || !d_y || epilogue < LAC_MODEL_OUT_BF16 || epilogue > LAC_MODEL_OUT_F32 ||
+        (epilogue == LAC_MODEL_OUT_BF16_ADD && !d_res) || (((uintptr_t)d_x | (uintptr_t)d_w | (uintptr_t)d_y |
+                                                             (uintptr_t)d_res) & 15))
+        return fail(LAC_E_ARG, "lac_model_gemm: bad argument");
+    if (!lac::model_gemm_shape_ok(M, N, K))
+        return fail(LAC_E_ARG, "lac_model_gemm: unsupported shape M=%lld N=%d K=%d (N %% 128 == 0, K %% 64 == 0, M >= 1)",
+                    (long long)M, N, K);
+    CK(lac::launch_model_gemm(d_x, d_w, M, N, K, epilogue, d_res, d_y, (cudaStream_t)stream), "lac_model_gemm");
+    return LAC_OK;
+}
+
+int lac_model_rmsnorm(const void* d_x, int64_t rows, int32_t dim, float eps, void* d_y, void* stream) {
+    if (!d_x || !d_y || rows < 0 || dim < 256 || dim % 256 || !(eps >= 0.f) || (((uintptr_t)d_x | (uintptr_t)d_y) & 15))
+        return fail(LAC_E_ARG, "lac_model_rmsnorm: bad argument (dim %d must be a positive multiple of 256)", dim);
+    if (rows == 0) return LAC_OK;
+    CK(lac::launch_model_rmsnorm(d_x, rows, dim, eps, d_y, (cudaStream_t)stream), "lac_model_rmsnorm");
+    return LAC_OK;
+}
+
+int lac_model_rope_kv(void* d_qkv, int64_t rows, int32_t n_streams, int32_t heads, int32_t kv_heads, int32_t hd,
+                      const void* d_cos, const void* d_sin, const int64_t* d_pos, int64_t p0, void* d_kc, void* d_vc,
+                      int32_t max_len, void* stream) {
+    if (!d_qkv || !d_cos || !d_sin || !d_kc || !d_vc || n_streams < 1 || rows < 0 || rows % n_streams ||
+        kv_heads < 1 || heads < kv_heads || heads % kv_heads || hd < 2 || hd % 2 || max_len < 1 || p0 < 0 ||
+        (!d_pos && p0 + rows / n_streams > max_len))
+        return fail(LAC_E_ARG, "lac_model_rope_kv: bad argument");
+    if (rows == 0) return LAC_OK;
+    CK(lac::launch_model_rope_kv(d_qkv, rows, n_streams, heads, kv_heads, hd, d_cos, d_sin, d_pos, p0, d_kc, d_vc,
+                                 max_len, (cudaStream_t)stream),
+       "lac_model_rope_kv");
+    return LAC_OK;
+}
+
+int lac_model_swiglu(const void* d_h, int64_t rows, int32_t ffn, void* d_y, void* stream) {
+    if (!d_h || !d_y || rows < 0 || ffn < 1) return fail(LAC_E_ARG, "lac_model_swiglu: bad argument");
+    if (rows == 0) return LAC_OK;
+    CK(lac::launch_model_swiglu(d_h, rows, ffn, d_y, (cudaStream_t)stream), "lac_model_swiglu");
+    return LAC_OK;
+}
+
+int lac_model_attention(const void* d_qkv, int32_t n_streams, int32_t n_q, int32_t heads, int32_t kv_heads, int32_t hd,
+                        const int64_t* d_pos, int64_t p0, const void* d_kc, const void* d_vc, int32_t max_len,
+                        void* d_out, void* stream) {
+    if (!d_qkv || !d_kc || !d_vc || !d_out || n_streams < 1 || n_q < 0 || kv_heads < 1 || heads < kv_heads ||
+        heads % kv_heads || heads / kv_heads > 64 || max_len < 1 || p0 < 0 || (!d_pos && p0 + n_q > max_len) ||
+        (((uintptr_t)d_qkv | (uintptr_t)d_kc | (uintptr_t)d_vc | (uintptr_t)d_out) & 15))
+        return fail(LAC_E_ARG, "lac_model_attention: bad argument");
+    if (hd != 64 && hd != 128) return fail(LAC_E_ARG, "lac_model_attention: head dim %d is not 64 or 128", hd);
+    if (n_q == 0) return LAC_OK;
+    CK(lac::launch_model_attention(d_qkv, n_streams, n_q, heads, kv_heads, hd, d_pos, p0, d_kc, d_vc, max_len, d_out,
+                                   (cudaStream_t)stream),
+       "lac_model_attention");
+    return LAC_OK;
+}
+
 int lac_encode_logits_host(const float* h_logits, const int32_t* h_syms, int64_t n_streams, int64_t T,
                            int32_t vocab, uint8_t* h_out, int64_t out_stride, uint64_t* h_nbits, int prec) {
     if ((T > 0 && (!h_logits || !h_syms)) || !h_out || !h_nbits || n_streams < 0 || T < 0 || out_stride < 1)

@@ -103,4 +103,17 @@ cudaError_t launch_table_decode(const Model&, int64_t n, int64_t T, const int32_
                                 const uint8_t* bytes, const int64_t* offsets, int32_t* syms, int64_t sym_stride,
                                 int P, cudaStream_t);
 
+// model_kernels.cu
+bool model_gemm_shape_ok(int64_t M, int N, int K);
+cudaError_t launch_model_gemm(const void* x, const void* w, int64_t M, int N, int K, int epi, const void* res, void* y,
+                              cudaStream_t st);
+cudaError_t launch_model_rmsnorm(const void* x, int64_t rows, int dim, float eps, void* y, cudaStream_t st);
+cudaError_t launch_model_rope_kv(void* qkv, int64_t rows, int S, int H, int KV, int hd, const void* cosb,
+                                 const void* sinb, const int64_t* d_pos, int64_t p0, void* kc, void* vc, int max_len,
+                                 cudaStream_t st);
+cudaError_t launch_model_swiglu(const void* h, int64_t rows, int F, void* y, cudaStream_t st);
+cudaError_t launch_model_attention(const void* qkv, int S, int n_q, int H, int KV, int hd, const int64_t* d_pos,
+                                   int64_t p0, const void* kc, const void* vc, int max_len, void* out,
+                                   cudaStream_t st);
+
 }  // namespace lac

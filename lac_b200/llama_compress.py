@@ -15,7 +15,12 @@ Losslessness needs bit-identical logits when compressing and decompressing.  The
 evaluating llama.cpp token by token in both directions; here both directions replay the SAME captured CUDA graph
 of `model.step` with the same batch shape (chunks are coded in batches of exactly `batch_streams` streams), so
 the same kernels run in the same order whether a file is written on one GPU and read on eight or the other way
-round.  (A prefill-style encoder would be faster but is not bit-reproducible against a stepwise decoder.)
+round.
+
+With LlamaModel(..., batch_invariant=True) the model runs the batch-invariant kernels of liblac_b200.so (DESIGN.md
+section 13): a row's logits do not depend on how many rows or positions a launch covers, so the encoder computes a
+whole block of positions in one prefill pass (StepEngine.prefill_encode_batch) and the stepwise decoder still
+reproduces its logits bit for bit.
 
 The per-token step -- model forward, LQ32 row summaries, fused symbol-range + range-coder kernel (or the decoder's
 serial pass), position update -- is ONE CUDA graph replay with no host-fed inputs: the tokens of the step are
@@ -73,12 +78,18 @@ _BUCKETS = (128, 256, 512, 1024, 2048, 4096, 8192)
 class LlamaModel(torch.nn.Module):
     """Llama-style decoder (RMSNorm, rotary GQA attention with a KV cache, SwiGLU), random-init, bf16 weights.
     step(tokens int64 [S]) -> fp32 logits [S, vocab] for the next position; the position lives on the device.
-    All shapes are static for a given attention bucket, so a step can be captured into a CUDA graph."""
+    All shapes are static for a given attention bucket, so a step can be captured into a CUDA graph.
+
+    batch_invariant=True runs every layer on the lac_model_* kernels instead of torch ops (same weights, same
+    function up to rounding), and adds prefill(): logits of a whole block of positions whose bits equal step()'s."""
 
     def __init__(self, cfg: LlamaConfig, n_streams: int, max_len: Optional[int] = None, seed: int = 0,
-                 device="cuda", dtype=torch.bfloat16):
+                 device="cuda", dtype=torch.bfloat16, batch_invariant: bool = False):
         super().__init__()
         self.cfg, self.S = cfg, int(n_streams)
+        self.batch_invariant = bool(batch_invariant)
+        if self.batch_invariant and dtype != torch.bfloat16:
+            raise ValueError("the batch-invariant kernels are bf16")
         self.max_len = int(max_len or cfg.max_len)
         self.device, self.dtype = torch.device(device), dtype
         g = torch.Generator(device=self.device).manual_seed(seed)
@@ -105,6 +116,10 @@ class LlamaModel(torch.nn.Module):
         self.pos = torch.zeros(1, dtype=torch.int64, device=self.device)
         self.ar = torch.arange(self.max_len, device=self.device)
 
+    def describe(self) -> str:
+        """The predictor configuration a file records (its LACB model tag): the two modes round differently."""
+        return self.cfg.describe() + (":bi" if self.batch_invariant else "")
+
     def reset(self):
         self.pos.zero_()
 
@@ -123,6 +138,8 @@ class LlamaModel(torch.nn.Module):
         attention is torch's scaled_dot_product_attention over the KV-cache slice with a position mask (measured
         against a bmm formulation and flash_attn_with_kvcache in tools/attn_bench.py: 0.10 vs 0.29 / 0.19 ms per
         layer at 256 streams x 2048 positions, deterministic)."""
+        if self.batch_invariant:
+            return self._forward_bi(tokens, self.pos, 0, 1)
         cfg, S, hd = self.cfg, self.S, self.hd
         H, K = cfg.heads, cfg.kv_heads
         pos = self.pos
@@ -142,6 +159,63 @@ class LlamaModel(torch.nn.Module):
             h13 = self._norm(x) @ self.w13[l]
             x = x + (torch.nn.functional.silu(h13[:, :cfg.ffn]) * h13[:, cfg.ffn:]) @ self.w2[l]
         return (self._norm(x) @ self.head).float()
+
+    @torch.no_grad()
+    def prefill(self, tokens: torch.Tensor, p0: int) -> torch.Tensor:
+        """tokens [T_blk, S] (position-major: row t holds every stream's input at position p0 + t) -> fp32 logits
+        [T_blk, S, vocab].  Writes the KV cache at positions p0 .. p0 + T_blk - 1 and leaves `pos` alone.  Row
+        (t, s) equals, bit for bit, what step() returns for stream s at position p0 + t after the same inputs."""
+        if not self.batch_invariant:
+            raise ValueError("prefill() needs LlamaModel(..., batch_invariant=True)")
+        Tb, S = tokens.shape
+        if S != self.S or p0 < 0 or p0 + Tb > self.max_len:
+            raise ValueError(f"prefill block [{Tb}, {S}] at p0={p0} does not fit [*, {self.S}] x {self.max_len}")
+        return self._forward_bi(tokens.reshape(-1), None, int(p0), Tb).view(Tb, S, self.cfg.vocab)
+
+    def _forward_bi(self, tokens, d_pos, p0, n_q):
+        """The model on the lac_model_* kernels over n_q positions x S streams (rows position-major)."""
+        cfg, S, hd = self.cfg, self.S, self.hd
+        H, K, d, M = cfg.heads, cfg.kv_heads, cfg.dim, n_q * self.S
+        L, st = _ffi.lib(), torch.cuda.current_stream(self.device).cuda_stream
+        pos_p = d_pos.data_ptr() if d_pos is not None else None
+        x = self.emb.index_select(0, tokens)
+        h = torch.empty_like(x)
+        qkv = torch.empty((M, (H + 2 * K) * hd), device=self.device, dtype=self.dtype)
+        o = torch.empty((M, H * hd), device=self.device, dtype=self.dtype)
+        h13 = torch.empty((M, 2 * cfg.ffn), device=self.device, dtype=self.dtype)
+        f = torch.empty((M, cfg.ffn), device=self.device, dtype=self.dtype)
+        logits = torch.empty((M, cfg.vocab), device=self.device, dtype=torch.float32)
+
+        def gemm(a, w, epi, y, res=None):
+            _ffi.check(L.lac_model_gemm(a.data_ptr(), w.data_ptr(), M, w.shape[1], w.shape[0], epi,
+                                        None if res is None else res.data_ptr(), y.data_ptr(), st))
+
+        def norm(a, y):
+            _ffi.check(L.lac_model_rmsnorm(a.data_ptr(), M, d, 1e-6, y.data_ptr(), st))
+        for l in range(cfg.layers):
+            norm(x, h)
+            gemm(h, self.wqkv[l], _ffi.LAC_MODEL_OUT_BF16, qkv)
+            _ffi.check(L.lac_model_rope_kv(qkv.data_ptr(), M, S, H, K, hd, self.cos.data_ptr(), self.sin.data_ptr(),
+                                           pos_p, p0, self.kc[l].data_ptr(), self.vc[l].data_ptr(), self.max_len, st))
+            _ffi.check(L.lac_model_attention(qkv.data_ptr(), S, n_q, H, K, hd, pos_p, p0, self.kc[l].data_ptr(),
+                                             self.vc[l].data_ptr(), self.max_len, o.data_ptr(), st))
+            gemm(o, self.wo[l], _ffi.LAC_MODEL_OUT_BF16_ADD, x, res=x)
+            norm(x, h)
+            gemm(h, self.w13[l], _ffi.LAC_MODEL_OUT_BF16, h13)
+            _ffi.check(L.lac_model_swiglu(h13.data_ptr(), M, cfg.ffn, f.data_ptr(), st))
+            gemm(f, self.w2[l], _ffi.LAC_MODEL_OUT_BF16_ADD, x, res=x)
+        norm(x, h)
+        gemm(h, self.head, _ffi.LAC_MODEL_OUT_F32, logits)
+        return logits
+
+
+# Logits of one prefill block (fp32 [T_blk, S, vocab]) stay within this many bytes: T_blk = budget // (4 S vocab).
+PREFILL_LOGITS_BYTES = 1 << 31
+
+
+def prefill_block(model: "LlamaModel") -> int:
+    """Positions per prefill block for this model's batch shape."""
+    return max(1, PREFILL_LOGITS_BYTES // (4 * model.S * model.cfg.vocab))
 
 
 def _bucket_for(pos: int, max_len: int) -> int:
@@ -199,7 +273,8 @@ class StepEngine:
         self.stream.wait_stream(cur)
         with torch.cuda.stream(self.stream):
             for t in range(n_steps):
-                bucket = _bucket_for(t, self.m.max_len)
+                # the batch-invariant attention reads the position itself: one graph per direction
+                bucket = self.m.max_len if self.m.batch_invariant else _bucket_for(t, self.m.max_len)
                 if not self.use_graphs:
                     fn(bucket)
                     continue
@@ -247,6 +322,35 @@ class StepEngine:
         self.enc.finish()
         return self.enc.bitstreams()
 
+    def prefill_encode_batch(self, tokens: np.ndarray, ntok: np.ndarray):
+        """encode_batch through model.prefill (batch-invariant models): the chunk in blocks of prefill_block()
+        positions, one prefill and one encode call per block.  The same bitstreams as encode_batch."""
+        S, T, V = self.m.S, self.T, self.m.cfg.vocab
+        assert tokens.shape == (S, T) and ntok.shape == (S,)
+        self.tok.copy_(torch.from_numpy(np.ascontiguousarray(tokens, dtype=np.int32)))
+        self.ntok.copy_(torch.from_numpy(np.ascontiguousarray(ntok, dtype=np.int32)))
+        if self.enc is None:
+            self.enc = coder.StreamEncoder(S, prec=self.prec, capacity_bytes=self.cap, device=self.m.device)
+        else:
+            self.enc.reset()
+        self.m.reset()
+        n = int(ntok.max()) if len(ntok) else 0
+        tb = prefill_block(self.m)
+        L, st = _ffi.lib(), torch.cuda.current_stream(self.m.device).cuda_stream
+        inp = torch.cat([torch.full((S, 1), BOS, dtype=torch.int64, device=self.m.device),
+                         self.tok[:, :T - 1].to(torch.int64)], 1)        # the model's input at every position
+        ws = coder.Workspace(S * tb, V, self.m.device)
+        for p0 in range(0, n, tb):
+            nb = min(tb, n - p0)
+            logits = self.m.prefill(inp[:, p0:p0 + nb].t().contiguous(), p0)
+            cnt = (self.ntok - p0).clamp_(0, nb).to(torch.int32)
+            _ffi.check(L.lac_ac_encode_logits_f32(logits.data_ptr(), S, nb, V, S * V, V, self.tok[:, p0:].data_ptr(),
+                                                  T, cnt.data_ptr(), self.enc.state.data_ptr(),
+                                                  self.enc.out.data_ptr(), self.cap, 0, self.prec, ws.ptr, ws.nbytes,
+                                                  st))
+        self.enc.finish()
+        return self.enc.bitstreams()
+
     def decode_batch(self, streams: List[bytes], ntok: np.ndarray) -> np.ndarray:
         S = self.m.S
         assert len(streams) == S and ntok.shape == (S,)
@@ -274,15 +378,16 @@ class LlamaCompressor:
         self.model, self.chunk, self.prec, self.group = model, int(chunk_tokens), int(prec), group
         self.vocab = model.cfg.vocab
         self.engine = StepEngine(model, chunk_tokens, prec, use_graphs)
-        self.tag = container.model_tag(model.cfg.describe())
+        self.tag = container.model_tag(model.describe())
 
     def compress(self, tokens) -> Optional[bytes]:
         toks = np.ascontiguousarray(tokens, dtype=np.int32)
         if toks.size and (int(toks.min()) < 0 or int(toks.max()) >= self.vocab):
             bad = int(toks.max()) if int(toks.max()) >= self.vocab else int(toks.min())
             raise AssertionError("unknown symbol", bad)  # llama_compress.py:51-52
-        return sharding.compress_sharded(toks, self.chunk, self.model.S, self.engine.encode_batch, self.prec,
-                                         self.vocab, self.model.device, self.tag, self.group)
+        encode = self.engine.prefill_encode_batch if self.model.batch_invariant else self.engine.encode_batch
+        return sharding.compress_sharded(toks, self.chunk, self.model.S, encode, self.prec, self.vocab,
+                                         self.model.device, self.tag, self.group)
 
     def decompress(self, blob: bytes, start: Optional[int] = None, stop: Optional[int] = None) -> Optional[np.ndarray]:
         """The tokens of the file, or tokens[start:stop] (0 <= start <= stop <= total, no negative indices): only
