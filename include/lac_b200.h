@@ -258,14 +258,16 @@ int lac_acs_decode_adaptive(int64_t *d_counts, int32_t vocab, int64_t inc, int64
  * Activations are position-major: row r = t * S + s is stream s at position base + t, where base = *d_pos when
  * d_pos (device, one int64) is given -- the per-token step, so one CUDA graph serves every position -- and p0
  * otherwise.  The KV cache is [S, kv_heads, max_len, hd] bf16; qkv rows are [heads | kv_heads | kv_heads] x hd.
+ * A launch with S = n streams may run on the first n streams of a larger cache (they are a prefix of it).
  * ---------------------------------------------------------------------------------- */
 #define LAC_MODEL_OUT_BF16 0      /* y = bf16(x @ w) */
 #define LAC_MODEL_OUT_BF16_ADD 1  /* y = bf16(res + bf16(x @ w)); y may be res */
 #define LAC_MODEL_OUT_F32 2       /* y = x @ w in fp32 (the logits) */
 
-/* Y[M, N] = X[M, K] @ W[K, N] on tcgen05 (TMA ring, accumulator in tensor memory), tile 128 x 128 x 64 for every
- * shape, K in one ascending pass.  N a multiple of 128 and K a multiple of 64 (every CONFIGS geometry); other
- * shapes return LAC_E_ARG.  All pointers 16-byte aligned. */
+/* Y[M, N] = X[M, K] @ W[K, N] on tcgen05 (TMA ring, accumulator in tensor memory), tile 128 x 128 x 64 (M <= 128:
+ * 128 x 64 x 64 with a deeper ring when N / 64 CTAs fit one wave; the same bits per row), K in one ascending pass.
+ * N a multiple of 128 and K a multiple of 64 (every CONFIGS geometry); other shapes return LAC_E_ARG.  All pointers
+ * 16-byte aligned. */
 int lac_model_gemm(const void *d_x, const void *d_w, int64_t M, int32_t N, int32_t K, int epilogue,
                    const void *d_res, void *d_y, void *stream);
 /* y = bf16(x * rsqrt(mean(x^2) + eps)) per row; dim a multiple of 256. */

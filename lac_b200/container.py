@@ -15,7 +15,9 @@ Layout (little endian):
     16  8  number of chunks N
     24  8  total tokens
     32  4  streams per model batch (chunks are coded in batches of exactly this many streams, the last batch padded
-           with empty streams, so the predictor sees the same batch shape when decoding -- on any number of GPUs)
+           with empty streams, so the predictor sees the same batch shape when decoding -- on any number of GPUs).
+           It binds torch-mode files only: a batch-invariant predictor's file (model tag of a `:bi` configuration)
+           decodes at any batch size, and there the field is informational
     36  4  model tag (CRC-32 of the predictor's configuration string; 0 = unspecified)
     40  N x (uint32 tokens in chunk, uint32 bits in chunk)      -- the index
     ..  chunk payloads, each byte aligned ((bits + 7) // 8 bytes), in chunk order

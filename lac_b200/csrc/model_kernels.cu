@@ -3,8 +3,11 @@
 //
 // The bits of output row r depend only on row r's inputs, the weights and (attention) the KV cache up to the row's
 // position -- never on M, on how many query positions a launch covers, or on which CTA or tile row computes it:
-//   * GEMM: tile 128 x 128 x 64 for every shape, K walked from 0 upwards in one accumulator, no split-K, no atomics.
-//     A row's MMAs read its own A row and the same B tiles in the same order whatever M is.
+//   * GEMM: tile 128 x 128 x 64 with a 3-stage ring; launches of M <= 128 whose 64-wide N tiles fit one wave use
+//     128 x 64 x 64 tiles with an 8-stage ring (twice the CTAs, more weight bytes in flight).  K walked from 0
+//     upwards in one accumulator, no split-K, no atomics.  A row's MMAs read its own A row and the same B columns in
+//     the same K order whatever M is; that a 128 x 64 MMA gives an element the bits of the 128 x 128 one is checked
+//     on the B200 (tests/test_gpu_any_batch.py).
 //   * RMSNorm: one warp per row, a fixed per-lane order over the row, then a fixed xor butterfly.
 //   * RoPE / SwiGLU: elementwise.
 //   * attention: every query visits 64-key blocks from slot 0 upwards with an fp32 online softmax (exp2); a block
@@ -22,8 +25,13 @@ namespace lac {
 namespace {
 
 constexpr int kBM = 128, kBN = 128, kBK = 64, kStages = 3;
-constexpr int kTileA = kBM * kBK * 2, kTileB = kBK * kBN * 2, kStage = kTileA + kTileB;  // bytes
-constexpr int kGemmSmem = kStages * kStage + 1024;                                        // + 1024-byte alignment slack
+constexpr int kSmallBN = 64, kSmallStages = 8;   // launches of M <= kBM: one tile row, so more and deeper N tiles
+constexpr int kTileA = kBM * kBK * 2;            // bytes
+constexpr int kAtomB = kBK * 64 * 2;             // one 64 x 64 B atom (64 columns of the 128-byte swizzle), bytes
+template <int BN> __host__ __device__ constexpr int tile_b() { return kBK * BN * 2; }
+template <int BN, int STAGES>  // + 1024-byte alignment slack
+__host__ __device__ constexpr int gemm_smem() { return STAGES * (kTileA + tile_b<BN>()) + 1024; }
+static_assert(gemm_smem<kSmallBN, kSmallStages>() <= 227 * 1024, "small-M ring exceeds the shared-memory limit");
 
 // ------------------------------------------------------------------ tcgen05 / TMA helpers
 __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
@@ -37,15 +45,18 @@ __device__ __forceinline__ uint64_t sdesc(uint32_t saddr, uint32_t lbo, uint32_t
     return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)((lbo >> 4) & 0x3FFF) << 16) |
            ((uint64_t)((sbo >> 4) & 0x3FFF) << 32) | (1ull << 46) | (2ull << 61);
 }
-// kind::f16 instruction descriptor: D fp32, A and B bf16, A K-major, B MN-major (W is [K, N] row-major), M x N
-constexpr uint32_t kIdesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((uint32_t)(kBN >> 3) << 17) |
-                            ((uint32_t)(kBM >> 4) << 24);
+// kind::f16 instruction descriptor: D fp32, A and B bf16, A K-major, B MN-major (W is [K, N] row-major), M x BN
+template <int BN>
+__host__ __device__ constexpr uint32_t idesc() {
+    return (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(kBM >> 4) << 24);
+}
 
+template <int BN>
 __device__ __forceinline__ void umma(uint32_t tmem, uint64_t a, uint64_t b, uint32_t accum) {
     asm volatile(
         "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem),
-        "l"(a), "l"(b), "r"(kIdesc), "r"(accum));
+        "l"(a), "l"(b), "r"(idesc<BN>()), "r"(accum));
 }
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -72,22 +83,23 @@ __device__ __forceinline__ float2 unpack_bf16(uint32_t v) {
 
 // ------------------------------------------------------------------ GEMM  Y[M, N] = X[M, K] @ W[K, N]
 // 128 threads: thread 0 feeds the smem ring by TMA, thread 32 issues the MMAs, warp 2 owns the tensor memory; then
-// the four warps drain the 128 x 128 fp32 accumulator (warp w: TMEM lanes = tile rows 32w .. 32w + 31).
-template <int EPI>
+// the four warps drain the 128 x BN fp32 accumulator (warp w: TMEM lanes = tile rows 32w .. 32w + 31).
+template <int EPI, int BN, int STAGES>
 __global__ void __launch_bounds__(128) gemm_kernel(const __grid_constant__ CUtensorMap ma,
                                                    const __grid_constant__ CUtensorMap mb, int64_t M, int N, int K,
                                                    const __nv_bfloat16* __restrict__ res, void* __restrict__ y) {
+    constexpr int kTileB = tile_b<BN>(), kStage = kTileA + kTileB;
     extern __shared__ uint8_t dsm[];
-    __shared__ uint64_t full[kStages], empty[kStages], done;
+    __shared__ uint64_t full[STAGES], empty[STAGES], done;
     __shared__ uint32_t tmem_slot;
     uint8_t* ring = (uint8_t*)(((uintptr_t)dsm + 1023) & ~(uintptr_t)1023);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n0 = blockIdx.x * kBN;
+    const int n0 = blockIdx.x * BN;
     const int m0 = blockIdx.y * kBM;
     const int nk = K / kBK;
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < kStages; ++s) {
+        for (int s = 0; s < STAGES; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], 1);
         }
@@ -96,7 +108,7 @@ __global__ void __launch_bounds__(128) gemm_kernel(const __grid_constant__ CUten
     }
     if (warp == 2) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)),
-                     "r"(kBN)
+                     "r"(BN)
                      : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
@@ -107,26 +119,26 @@ __global__ void __launch_bounds__(128) gemm_kernel(const __grid_constant__ CUten
 
     if (threadIdx.x == 0) {  // producer
         for (int kb = 0; kb < nk; ++kb) {
-            const int s = kb % kStages;
-            if (kb >= kStages) mbar_wait(&empty[s], ((kb / kStages) - 1) & 1);
+            const int s = kb % STAGES;
+            if (kb >= STAGES) mbar_wait(&empty[s], ((kb / STAGES) - 1) & 1);
             uint8_t* a = ring + s * kStage;
             uint8_t* b = a + kTileA;
             mbar_expect_tx(&full[s], kStage);
             tma_load_2d(a, &ma, kb * kBK, m0, &full[s]);
-            tma_load_2d(b, &mb, n0, kb * kBK, &full[s]);
-            tma_load_2d(b + kTileB / 2, &mb, n0 + 64, kb * kBK, &full[s]);
+#pragma unroll
+            for (int j = 0; j < BN / 64; ++j) tma_load_2d(b + j * kAtomB, &mb, n0 + 64 * j, kb * kBK, &full[s]);
         }
     } else if (threadIdx.x == 32) {  // MMA issuer
         for (int kb = 0; kb < nk; ++kb) {
-            const int s = kb % kStages;
-            mbar_wait(&full[s], (kb / kStages) & 1);
+            const int s = kb % STAGES;
+            mbar_wait(&full[s], (kb / STAGES) & 1);
             tc_fence_after();
             const uint32_t a = smem_u32(ring + s * kStage), b = a + kTileA;
 #pragma unroll
             for (int k = 0; k < kBK / 16; ++k) {
                 // A: K-major, 8-row groups 1024 B apart, +32 B per 16 K.  B: MN-major, 64-column atoms 8 KB apart,
                 // 8-K-row groups 1024 B apart, +2048 B per 16 K.
-                umma(tmem, sdesc(a + k * 32, 16, 1024), sdesc(b + k * 2048, kTileB / 2, 1024), (kb | k) != 0);
+                umma<BN>(tmem, sdesc(a + k * 32, 16, 1024), sdesc(b + k * 2048, kAtomB, 1024), (kb | k) != 0);
             }
             umma_commit(&empty[s]);
         }
@@ -139,7 +151,7 @@ __global__ void __launch_bounds__(128) gemm_kernel(const __grid_constant__ CUten
     const int64_t row = (int64_t)m0 + warp * 32 + lane;
     const bool live = row < M;
 #pragma unroll 1
-    for (int c = 0; c < kBN; c += 16) {
+    for (int c = 0; c < BN; c += 16) {
         uint32_t r[16];
         tmem_ld16(tmem + ((uint32_t)(warp * 32) << 16) + c, r);
         if (!live) continue;
@@ -171,7 +183,8 @@ __global__ void __launch_bounds__(128) gemm_kernel(const __grid_constant__ CUten
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kBN) : "memory");
+    if (warp == 2)
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(BN) : "memory");
 }
 
 typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -204,18 +217,44 @@ bool make_map(CUtensorMap* m, const void* p, int64_t inner, int64_t outer, uint3
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int EPI>
+template <int EPI, int BN, int STAGES>
 cudaError_t gemm_launch(const CUtensorMap& ma, const CUtensorMap& mb, int64_t M, int N, int K, const void* res,
                         void* y, cudaStream_t st) {
+    constexpr int smem = gemm_smem<BN, STAGES>();
     static bool attr = false;
     if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(gemm_kernel<EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemmSmem);
+        cudaError_t e =
+            cudaFuncSetAttribute(gemm_kernel<EPI, BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return e;
         attr = true;
     }
-    dim3 grid(N / kBN, (unsigned)((M + kBM - 1) / kBM));
-    gemm_kernel<EPI><<<grid, 128, kGemmSmem, st>>>(ma, mb, M, N, K, (const __nv_bfloat16*)res, y);
+    dim3 grid(N / BN, (unsigned)((M + kBM - 1) / kBM));
+    gemm_kernel<EPI, BN, STAGES><<<grid, 128, smem, st>>>(ma, mb, M, N, K, (const __nv_bfloat16*)res, y);
     return cudaGetLastError();
+}
+
+int sm_count() {
+    static int n = 0;
+    if (!n) {
+        int dev = 0;
+        if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) !=
+                                                      cudaSuccess)
+            n = 1;
+    }
+    return n;
+}
+
+// M <= 128 is one tile row, so a 128-wide N tile leaves N / 128 CTAs (16 for a 2048-wide weight) each walking all of
+// K: the step is bound by the weight loads those few SMs keep in flight.  64-wide tiles double the CTAs and the
+// 8-stage ring keeps 8 K-steps of each in flight -- as long as they fit one wave: past the SM count (w13 and the
+// head of `1b`) the 197 KB ring allows one CTA per SM against two of the 3-stage one, and the wide tile is faster.
+// A row gets the same bits from either tile.
+template <int EPI>
+cudaError_t gemm_dispatch(const CUtensorMap& ma, const CUtensorMap& mb, int64_t M, int N, int K, const void* res,
+                          void* y, cudaStream_t st) {
+    if (M <= kBM && N / kSmallBN <= sm_count())
+        return gemm_launch<EPI, kSmallBN, kSmallStages>(ma, mb, M, N, K, res, y, st);
+    return gemm_launch<EPI, kBN, kStages>(ma, mb, M, N, K, res, y, st);
 }
 
 // ------------------------------------------------------------------ RMSNorm: one warp per row
@@ -476,9 +515,9 @@ cudaError_t launch_model_gemm(const void* x, const void* w, int64_t M, int N, in
     CUtensorMap ma, mb;
     if (!make_map(&ma, x, K, M, kBM) || !make_map(&mb, w, N, K, kBK)) return cudaErrorInvalidValue;
     switch (epi) {
-        case LAC_MODEL_OUT_BF16: return gemm_launch<LAC_MODEL_OUT_BF16>(ma, mb, M, N, K, res, y, st);
-        case LAC_MODEL_OUT_BF16_ADD: return gemm_launch<LAC_MODEL_OUT_BF16_ADD>(ma, mb, M, N, K, res, y, st);
-        default: return gemm_launch<LAC_MODEL_OUT_F32>(ma, mb, M, N, K, res, y, st);
+        case LAC_MODEL_OUT_BF16: return gemm_dispatch<LAC_MODEL_OUT_BF16>(ma, mb, M, N, K, res, y, st);
+        case LAC_MODEL_OUT_BF16_ADD: return gemm_dispatch<LAC_MODEL_OUT_BF16_ADD>(ma, mb, M, N, K, res, y, st);
+        default: return gemm_dispatch<LAC_MODEL_OUT_F32>(ma, mb, M, N, K, res, y, st);
     }
 }
 

@@ -81,7 +81,9 @@ class LlamaModel(torch.nn.Module):
     All shapes are static for a given attention bucket, so a step can be captured into a CUDA graph.
 
     batch_invariant=True runs every layer on the lac_model_* kernels instead of torch ops (same weights, same
-    function up to rounding), and adds prefill(): logits of a whole block of positions whose bits equal step()'s."""
+    function up to rounding), and adds prefill(): logits of a whole block of positions whose bits equal step()'s.
+    In that mode step() and prefill() also take n <= S streams (the tokens' shape): they run on the first n slots of
+    the KV cache, and a stream's logits are the same bits whatever n is."""
 
     def __init__(self, cfg: LlamaConfig, n_streams: int, max_len: Optional[int] = None, seed: int = 0,
                  device="cuda", dtype=torch.bfloat16, batch_invariant: bool = False):
@@ -137,9 +139,15 @@ class LlamaModel(torch.nn.Module):
         """One position for all S streams; attends over the first `bucket` cache slots (bucket > pos).  The
         attention is torch's scaled_dot_product_attention over the KV-cache slice with a position mask (measured
         against a bmm formulation and flash_attn_with_kvcache in tools/attn_bench.py: 0.10 vs 0.29 / 0.19 ms per
-        layer at 256 streams x 2048 positions, deterministic)."""
+        layer at 256 streams x 2048 positions, deterministic).  Batch-invariant: tokens [n], 1 <= n <= S, streams
+        0 .. n - 1, logits [n, vocab]."""
         if self.batch_invariant:
+            n = tokens.shape[0]
+            if not 1 <= n <= self.S:
+                raise ValueError(f"step over {n} streams; this model holds 1 .. {self.S}")
             return self._forward_bi(tokens, self.pos, 0, 1)
+        if tokens.shape[0] != self.S:
+            raise ValueError(f"a torch-mode step runs exactly {self.S} streams, got {tokens.shape[0]}")
         cfg, S, hd = self.cfg, self.S, self.hd
         H, K = cfg.heads, cfg.kv_heads
         pos = self.pos
@@ -162,20 +170,23 @@ class LlamaModel(torch.nn.Module):
 
     @torch.no_grad()
     def prefill(self, tokens: torch.Tensor, p0: int) -> torch.Tensor:
-        """tokens [T_blk, S] (position-major: row t holds every stream's input at position p0 + t) -> fp32 logits
-        [T_blk, S, vocab].  Writes the KV cache at positions p0 .. p0 + T_blk - 1 and leaves `pos` alone.  Row
-        (t, s) equals, bit for bit, what step() returns for stream s at position p0 + t after the same inputs."""
+        """tokens [T_blk, n] (position-major: row t holds every stream's input at position p0 + t; n <= S streams)
+        -> fp32 logits [T_blk, n, vocab].  Writes the KV cache at positions p0 .. p0 + T_blk - 1 and leaves `pos`
+        alone.  Row (t, s) equals, bit for bit, what step() returns for stream s at position p0 + t after the same
+        inputs."""
         if not self.batch_invariant:
             raise ValueError("prefill() needs LlamaModel(..., batch_invariant=True)")
-        Tb, S = tokens.shape
-        if S != self.S or p0 < 0 or p0 + Tb > self.max_len:
-            raise ValueError(f"prefill block [{Tb}, {S}] at p0={p0} does not fit [*, {self.S}] x {self.max_len}")
-        return self._forward_bi(tokens.reshape(-1), None, int(p0), Tb).view(Tb, S, self.cfg.vocab)
+        Tb, n = tokens.shape
+        if not 1 <= n <= self.S or p0 < 0 or p0 + Tb > self.max_len:
+            raise ValueError(f"prefill block [{Tb}, {n}] at p0={p0} does not fit [*, <= {self.S}] x {self.max_len}")
+        return self._forward_bi(tokens.reshape(-1), None, int(p0), Tb).view(Tb, n, self.cfg.vocab)
 
     def _forward_bi(self, tokens, d_pos, p0, n_q):
-        """The model on the lac_model_* kernels over n_q positions x S streams (rows position-major)."""
-        cfg, S, hd = self.cfg, self.S, self.hd
-        H, K, d, M = cfg.heads, cfg.kv_heads, cfg.dim, n_q * self.S
+        """The model on the lac_model_* kernels over n_q positions x S streams (rows position-major), S the
+        tokens' stream count: the first S slots of the KV cache."""
+        cfg, hd = self.cfg, self.hd
+        S = tokens.numel() // n_q
+        H, K, d, M = cfg.heads, cfg.kv_heads, cfg.dim, tokens.numel()
         L, st = _ffi.lib(), torch.cuda.current_stream(self.device).cuda_stream
         pos_p = d_pos.data_ptr() if d_pos is not None else None
         x = self.emb.index_select(0, tokens)
@@ -225,9 +236,25 @@ def _bucket_for(pos: int, max_len: int) -> int:
     return max_len
 
 
+def active_streams(count: int, S: int) -> int:
+    """The stream count a batch-invariant decode of `count` streams runs at: the smallest rung >= count of the
+    ladder 1, 2, 4, ... (powers of two below S), S.  A fixed ladder bounds the graphs to about log2(S) + 1 per
+    direction."""
+    if not 1 <= count <= S:
+        raise ValueError(f"{count} streams do not fit a batch of {S}")
+    n = 1
+    while n < count:
+        n *= 2
+    return min(n, S)
+
+
 class StepEngine:
     """The per-token loop of one batch: holds the model, the static device buffers and one captured CUDA graph per
-    (direction, attention bucket).  A step is `graph.replay()`; nothing is fed from the host."""
+    (direction, attention bucket, active streams).  A step is `graph.replay()`; nothing is fed from the host.
+
+    A torch-mode model always runs its S streams.  A batch-invariant model decodes a batch of any size <= S at the
+    active stream count active_streams(): the first n rows of the buffers and of the KV cache, one decoder per n,
+    the workspace sized for S.  Its attention reads the position itself, so that is one graph per (direction, n)."""
 
     def __init__(self, model: LlamaModel, chunk_tokens: int, prec: int, use_graphs: bool = True):
         self.m, self.T, self.prec, self.use_graphs = model, int(chunk_tokens), int(prec), use_graphs
@@ -242,13 +269,15 @@ class StepEngine:
         self.cap = self.T * 8 + 64
         self.enc: Optional[coder.StreamEncoder] = None
         self.dec: Optional[coder.StreamDecoder] = None
+        self.decs: Dict[int, coder.StreamDecoder] = {}   # decoder per active stream count
+        self.n = S                                       # active streams of the batch being coded
         self.graphs: Dict = {}
         self.stream = torch.cuda.Stream(device=dev)
 
     # ---- one step, expressed on device tensors only
     def _prev_tokens(self):
         pos = self.m.pos
-        prev = self.tok.index_select(1, (pos - 1).clamp_(min=0)).squeeze(1).to(torch.int64)
+        prev = self.tok[:self.n].index_select(1, (pos - 1).clamp_(min=0)).squeeze(1).to(torch.int64)
         return torch.where(pos > 0, prev, torch.full_like(prev, BOS))
 
     def _enc_step(self, bucket):
@@ -260,11 +289,13 @@ class StepEngine:
         pos.add_(1)
 
     def _dec_step(self, bucket):
+        n = self.n
+        tok, live, sym = self.tok[:n], self.live[:n], self.sym[:n]
         logits = self.m.step(self._prev_tokens(), bucket)
         pos = self.m.pos
-        self.live.copy_((self.ntok > pos).to(torch.int32))
-        self.dec.decode_step(logits, self.live, self.ws, out=self.sym)
-        self.tok.index_copy_(1, pos, torch.where(self.live > 0, self.sym, torch.zeros_like(self.sym)).unsqueeze(1))
+        live.copy_((self.ntok[:n] > pos).to(torch.int32))
+        self.dec.decode_step(logits, live, self.ws, out=sym)
+        tok.index_copy_(1, pos, torch.where(live > 0, sym, torch.zeros_like(sym)).unsqueeze(1))
         pos.add_(1)
 
     def _run(self, kind, n_steps):
@@ -278,7 +309,7 @@ class StepEngine:
                 if not self.use_graphs:
                     fn(bucket)
                     continue
-                key = (kind, bucket)
+                key = (kind, bucket, self.n)
                 if key not in self.graphs:
                     # warm-up run outside capture (cuBLAS handles / workspaces), then rewind what it changed
                     snap = self._snapshot(kind)
@@ -309,7 +340,7 @@ class StepEngine:
 
     # ---- whole batches
     def encode_batch(self, tokens: np.ndarray, ntok: np.ndarray):
-        S = self.m.S
+        S = self.n = self.m.S
         assert tokens.shape == (S, self.T) and ntok.shape == (S,)
         self.tok.copy_(torch.from_numpy(np.ascontiguousarray(tokens, dtype=np.int32)))
         self.ntok.copy_(torch.from_numpy(np.ascontiguousarray(ntok, dtype=np.int32)))
@@ -352,13 +383,19 @@ class StepEngine:
         return self.enc.bitstreams()
 
     def decode_batch(self, streams: List[bytes], ntok: np.ndarray) -> np.ndarray:
-        S = self.m.S
-        assert len(streams) == S and ntok.shape == (S,)
-        self.ntok.copy_(torch.from_numpy(np.ascontiguousarray(ntok, dtype=np.int32)))
+        """Decode ntok[i] tokens of streams[i] -> int32 [len(streams), chunk_tokens].  A torch-mode model takes
+        exactly S streams; a batch-invariant one any 1 .. S, run at active_streams() with empty padding streams."""
+        S, B = self.m.S, len(streams)
+        assert ntok.shape == (B,) and (B == S or (self.m.batch_invariant and 1 <= B <= S))
+        n = self.n = active_streams(B, S) if self.m.batch_invariant else S
+        streams = list(streams) + [b""] * (n - B)
+        self.ntok.zero_()
+        self.ntok[:B].copy_(torch.from_numpy(np.ascontiguousarray(ntok, dtype=np.int32)))
         self.tok.zero_()
+        self.dec = self.decs.get(n)
         if self.dec is None:
-            self.dec = coder.StreamDecoder(streams, prec=self.prec, device=self.m.device,
-                                           capacity_bytes=S * self.cap)
+            self.dec = self.decs[n] = coder.StreamDecoder(streams, prec=self.prec, device=self.m.device,
+                                                          capacity_bytes=n * self.cap)
         else:
             self.dec.reset(streams)
         self.m.reset()
@@ -366,7 +403,7 @@ class StepEngine:
         st = self.dec.status()
         if st & _ffi.LAC_ST_TRUNC:
             raise _ffi.LacError(_ffi.LAC_E_STREAM, "truncated or foreign bitstream (wrong model for this file?)")
-        return self.tok.cpu().numpy()
+        return self.tok[:B].cpu().numpy()
 
 
 class LlamaCompressor:
@@ -390,18 +427,26 @@ class LlamaCompressor:
                                          self.model.device, self.tag, self.group)
 
     def decompress(self, blob: bytes, start: Optional[int] = None, stop: Optional[int] = None) -> Optional[np.ndarray]:
-        """The tokens of the file, or tokens[start:stop] (0 <= start <= stop <= total, no negative indices): only
-        the batches that hold the range are decoded, each for as many steps as its needed chunks reach into it."""
+        """The tokens of the file, or tokens[start:stop] (0 <= start <= stop <= total, no negative indices).
+
+        A torch-mode file decodes in the batches it was written in (the header's batch_streams must be this model's
+        S): only the batches that hold the range, each for as many steps as its needed chunks reach into it.  A file
+        written by this batch-invariant predictor (its tag ends in :bi) decodes at any S: only the needed chunks,
+        packed into batches of similar length (sharding.decompress_packed); its batch_streams is informational."""
         c = container.unpack(blob)
         if c.vocab != self.vocab or c.quantiser != container.QUANT_LQ32:
             raise ValueError("container was written for a different vocabulary / quantiser")
-        if c.batch_streams != self.model.S or c.chunk_tokens != self.chunk:
+        packed = self.model.batch_invariant and c.tag == self.tag
+        if (not packed and c.batch_streams != self.model.S) or c.chunk_tokens != self.chunk:
             raise ValueError(f"container was written with batches of {c.batch_streams} streams x {c.chunk_tokens} "
                              f"tokens; this compressor runs {self.model.S} x {self.chunk}")
         if c.tag and c.tag != self.tag:
             raise ValueError("container was written with a different predictor configuration")
-        return sharding.decompress_sharded(blob, self.engine.decode_batch, self.model.device, self.group,
-                                           0 if start is None else start, stop)
+        start = 0 if start is None else start
+        if packed:
+            return sharding.decompress_packed(blob, self.engine.decode_batch, self.model.S, self.model.device,
+                                              self.group, start, stop)
+        return sharding.decompress_sharded(blob, self.engine.decode_batch, self.model.device, self.group, start, stop)
 
 
 # ------------------------------------------------------------------ the reference's own entry points

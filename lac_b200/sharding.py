@@ -6,6 +6,10 @@ Chunks are coded in model batches of exactly `batch_streams` streams (the last b
 streams): the predictor then sees the same batch shape whether a file is written by 1 GPU and read by 8 or the
 other way round, which is what makes the logits -- and with them the decode -- bit-reproducible.  Batches, not
 chunks, are what is dealt to the ranks: rank r owns a contiguous range of batches.
+
+That batch shape binds torch-mode files only.  A batch-invariant predictor gives a stream the same logits in a
+batch of any size, so such a file is decoded chunk by chunk (decompress_packed): the needed chunks are packed into
+batches of the decoder's size and dealt over all ranks, whatever batch_streams the header records.
 """
 from __future__ import annotations
 
@@ -160,6 +164,21 @@ def _check_range(start, stop, total: int) -> Tuple[int, int]:
     return int(start), int(stop)
 
 
+def _plan(c: container.Container, start, stop) -> Tuple[np.ndarray, int, int]:
+    """(first token of every chunk and the total, start, stop) after the bounds check."""
+    first = np.zeros(c.n_chunks + 1, dtype=np.int64)
+    np.cumsum(c.ntok, out=first[1:])
+    start, stop = _check_range(start, first[-1] if stop is None else stop, int(first[-1]))
+    return first, start, stop
+
+
+def _want(c: container.Container, first: np.ndarray, start: int, stop: int) -> np.ndarray:
+    """Tokens to decode per chunk: the prefix up to stop of every chunk that overlaps [start, stop), else 0."""
+    want = np.minimum(c.ntok.astype(np.int64), np.maximum(stop - first[:-1], 0))
+    want[first[1:] <= start] = 0
+    return want
+
+
 def decompress_sharded(blob: bytes, decode_batch: DecodeBatch, device, group=None, start: int = 0,
                        stop: Optional[int] = None) -> Optional[np.ndarray]:
     """Every rank passes the SAME file and range; rank 0 returns tokens[start:stop] (None elsewhere).  The default
@@ -173,13 +192,10 @@ def decompress_sharded(blob: bytes, decode_batch: DecodeBatch, device, group=Non
     with no tokens overlaps no range and is never decoded."""
     rank, world = _world(group)
     c = container.unpack(blob)
-    first = np.zeros(c.n_chunks + 1, dtype=np.int64)          # first token of every chunk, and the total
-    np.cumsum(c.ntok, out=first[1:])
-    start, stop = _check_range(start, first[-1] if stop is None else stop, int(first[-1]))
+    first, start, stop = _plan(c, start, stop)
     if start == stop:
         return np.zeros(0, dtype=np.int32) if rank == 0 else None
-    want = np.minimum(c.ntok.astype(np.int64), np.maximum(stop - first[:-1], 0))   # tokens to decode per chunk
-    want[first[1:] <= start] = 0
+    want = _want(c, first, start, stop)
     needed = np.flatnonzero(want)
     B = c.batch_streams or max(c.n_chunks, 1)
     batches = np.unique(needed // B)
@@ -205,4 +221,63 @@ def decompress_sharded(blob: bytes, decode_batch: DecodeBatch, device, group=Non
         return None
     got = got.cpu().numpy()
     flat = np.concatenate([got[j, : want[i]] for j, i in enumerate(needed)])
+    return flat[start - first[needed[0]]:]
+
+
+def pack_batches(want: np.ndarray, batch_streams: int, world: int) -> List[np.ndarray]:
+    """The decode batches of a batch-invariant read: the chunks with want > 0, ordered by want descending (ties in
+    chunk order) so that short prefixes do not wait in a batch with long ones.
+      * More needed chunks than world x batch_streams: cut from the front into batches of batch_streams, so the
+        shortest prefixes share the last batch (which the decoder runs at a smaller active size).  With one rank
+        this is the least total of steps (the sum of every batch's longest prefix) any batching of <= S chunks
+        reaches.
+      * Otherwise: min(world, needed) balanced batches, none larger than ceil(needed / world) <= batch_streams,
+        so every rank gets work while there are chunks for it."""
+    needed = np.flatnonzero(want)
+    order = needed[np.argsort(-want[needed], kind="stable")]
+    if len(order) > world * batch_streams:
+        return [order[b:b + batch_streams] for b in range(0, len(order), batch_streams)]
+    n_batches = min(world, len(order))
+    return [order[b:e] for b, e in (chunk_range(len(order), k, n_batches) for k in range(n_batches))]
+
+
+def decompress_packed(blob: bytes, decode_batch: DecodeBatch, batch_streams: int, device, group=None,
+                      start: int = 0, stop: Optional[int] = None) -> Optional[np.ndarray]:
+    """decompress_sharded for a file of a batch-invariant predictor, whose rows do not depend on the batch they
+    share: every rank passes the SAME file and range and its decoder's stream count; rank 0 returns
+    tokens[start:stop] (None elsewhere).
+
+    Each chunk that overlaps the range is decoded exactly once from its first token, for min(its length, stop -
+    its first token) tokens.  pack_batches groups them into batches of at most batch_streams chunks, and batch k
+    goes to rank k % world (longest batches first, so round robin also balances the steps).  decode_batch gets
+    exactly the batch's streams; a batch costs as many model steps as its longest needed prefix.  The file's own
+    batch_streams plays no part."""
+    rank, world = _world(group)
+    c = container.unpack(blob)
+    first, start, stop = _plan(c, start, stop)
+    if start == stop:
+        return np.zeros(0, dtype=np.int32) if rank == 0 else None
+    want = _want(c, first, start, stop)
+    batches = pack_batches(want, int(batch_streams), world)
+    mine = batches[rank::world]
+    owned = [np.concatenate(batches[r::world]) if batches[r::world] else np.zeros(0, np.int64) for r in range(world)]
+    spans, at = [], 0
+    for o in owned:
+        spans.append((at, at + len(o)))
+        at += len(o)
+    off = c.offsets()
+    local = np.zeros((len(owned[rank]), c.chunk_tokens), dtype=np.int32)
+    at = 0
+    for ids in mine:
+        got = decode_batch([c.payload[off[i]:off[i + 1]] for i in ids], want[ids].astype(np.int32))
+        local[at:at + len(ids)] = got[: len(ids)]
+        at += len(ids)
+    got = gather_tokens(torch.from_numpy(local).to(device), spans[-1][1], c.chunk_tokens, spans, 0, group)
+    if rank != 0:
+        return None
+    got = got.cpu().numpy()
+    row = np.empty(c.n_chunks, dtype=np.int64)        # chunk -> its row in the gathered rank-order rows
+    row[np.concatenate(owned)] = np.arange(spans[-1][1])
+    needed = np.flatnonzero(want)
+    flat = np.concatenate([got[row[i], : want[i]] for i in needed])
     return flat[start - first[needed[0]]:]
